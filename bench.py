@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c3|c4]
     python bench.py --impl reference ...     # CPU arm (oracle port, all cores)
+    python bench.py ... --dump-outputs DIR    # also write the results as .npy
 
 BASELINE.json's metric has two halves.  The line's own metric/value is the
 first (batched fits/s, workload c2 = configs[1]); the default run also measures
@@ -188,6 +189,59 @@ def gpu_parity_of_cpu_sample(w, fun, jac, lb, ub, dev):
         "note": "GPU path vs the oracle on the cpu_baseline sample; the gates "
                 "(1e-8 on x / cost, equal status) are enforced in tests/",
     }
+
+
+# ------------------------------------------------------------ outputs -----
+
+# --dump-outputs keeps under 64 MB for every workload: at most this many
+# batched problems and tall rows, a fixed seeded sample of the larger outputs
+DUMP_PROBLEMS = 32768
+DUMP_ROWS = 8192
+
+
+def _sample(total, k):
+    """Sorted seeded sample of k of range(total); all of it when total <= k."""
+    if total <= k:
+        return np.arange(total)
+    return np.sort(np.random.default_rng(0).choice(total, k, replace=False))
+
+
+def write_outputs(out_dir, prefix, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if hasattr(a, "cpu"):
+            a = a.cpu().numpy()
+        np.save(os.path.join(out_dir, prefix + name + ".npy"),
+                np.asarray(a, dtype=np.float64))
+
+
+def dump_batched(out_dir, prefix, outs, chunk, B):
+    """Every per-problem field least_squares_batched returned in the last
+    timed step, for a seeded sample of the problems."""
+    import torch
+    idx = _sample(B, DUMP_PROBLEMS)
+    arrays = {"problem_index": idx}
+    for key in ("x", "obj_value", "optimality", "active_mask", "status",
+                "nfev", "njev", "fun"):
+        parts = []
+        for c, o in enumerate(outs):
+            c0 = c * chunk
+            sel = idx[(idx >= c0) & (idx < c0 + o.x.shape[0])] - c0
+            parts.append(o[key][torch.as_tensor(sel, device=o.x.device)].cpu())
+        arrays[key] = torch.cat(parts)
+    write_outputs(out_dir, prefix, arrays)
+
+
+def dump_tall(out_dir, prefix, res):
+    """The result of the last timed tall solve: x and the scalars whole, the
+    residual and the Jacobian on a seeded sample of the rows."""
+    import torch
+    rows = _sample(res.fun.shape[0], DUMP_ROWS)
+    r = torch.as_tensor(rows, device=res.fun.device)
+    write_outputs(out_dir, prefix, {
+        "x": res.x, "active_mask": res.active_mask, "obj_value": res.obj_value,
+        "optimality": res.optimality, "status": res.status, "nfev": res.nfev,
+        "njev": res.njev, "row_index": rows, "fun": res.fun[r], "jac": res.jac[r]})
 
 
 def static_config(w, B, chunk, callbacks=None):
@@ -482,11 +536,12 @@ def run_tall_reference_arm(args, w, standalone=True):
     return line
 
 
-def run_tall(args, w, standalone=True, light=False):
+def run_tall(args, w, standalone=True, light=False, dump_prefix=None):
     """Tall workload.  standalone: own process-group set-up and JSON line;
     otherwise called from the batched main (default run) which attaches the
     returned dict to its line as "tall".  light: value only (no e2e, no CPU
-    baseline) -- the asymmetric-start companion record."""
+    baseline) -- the asymmetric-start companion record.  dump_prefix: with
+    --dump-outputs, the last timed solve's result goes to DIR/<prefix>*.npy."""
     import torch
     import torch.distributed as dist
     from bounded_lsq_b200 import least_squares
@@ -555,6 +610,8 @@ def run_tall(args, w, standalone=True, light=False):
         barrier()
     dev_ms = reduce_max(e0.elapsed_time(e1))
     value = its / (dev_ms * 1e-3)
+    if args.dump_outputs and dump_prefix is not None and rank == 0:
+        dump_tall(args.dump_outputs, dump_prefix, res)
 
     # per-kernel timing (separate instrumented solve)
     collect = {}
@@ -708,12 +765,21 @@ def main():
                     help="tall workloads: override the method (C5: TRF vs dogbox)")
     ap.add_argument("--rows", type=int, default=None,
                     help="tall workload: total rows (default 2^24)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed "
+                         "to DIR/<name>.npy (float64; a seeded sample of the "
+                         "problems / rows, under 64 MB in all); the default run "
+                         "adds the tall solve as DIR/tall_<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's results (--impl b200)")
     w = WORKLOADS[args.workload]
     if w.get("kind") == "tall":
         if args.impl == "reference":
             return run_tall_reference_arm(args, w)
-        return run_tall(args, w)
+        return run_tall(args, w, dump_prefix="")
     if args.impl == "reference":
         return run_reference_arm(args, w)
 
@@ -730,29 +796,32 @@ def main():
         dist.init_process_group("nccl", device_id=dev)
 
     line = run_batched(args, w, args.workload, args.steps, args.warmup,
-                       args.batch or w["B"], cpu_baseline=not args.no_cpu_baseline)
+                       args.batch or w["B"], cpu_baseline=not args.no_cpu_baseline,
+                       dump_prefix="")
     if line is not None and pinned is not None:
         line["config"]["driver_thread_affinity"] = pinned
 
     # the other half of BASELINE.json's metric (TRF iterations/s at m=16M,
-    # n=64) rides along on the default run as the "tall" object, and a short
-    # run of configs[2] (C3: dogbox, 2-point Jacobian; ONE 1M-problem chunk of
-    # the 10M) as "c3".  Their headline numbers are repeated inside `config`.
+    # n=64) rides along on the default run as the "tall" object, and a run of
+    # configs[2] (C3: dogbox, 2-point Jacobian; ONE 1M-problem chunk of the
+    # 10M) as "c3".  Their headline numbers are repeated inside `config`.
+    # Every record times --steps steps after --warmup warm-up solves: a record
+    # of only two steps moved by 30% between runs whenever one host stall
+    # landed in it.
     if args.workload == "c2" and not args.no_tall and args.batch is None:
         torch.cuda.empty_cache()
-        tall_line = run_tall(args, WORKLOADS["c4"], standalone=False)
+        tall_line = run_tall(args, WORKLOADS["c4"], standalone=False, dump_prefix="tall_")
         torch.cuda.empty_cache()
         tall_asym = run_tall(args, dict(WORKLOADS["c4"], x0_tail=(0.8, 1.5, 0.3, 4.0)),
                              standalone=False, light=True)
         torch.cuda.empty_cache()
-        c3_line = run_batched(args, WORKLOADS["c3"], "c3", max(2, args.steps // 4),
-                              max(1, min(args.warmup, 2)), 1_000_000,
-                              cpu_baseline=False)
+        c3_line = run_batched(args, WORKLOADS["c3"], "c3", args.steps, args.warmup,
+                              1_000_000, cpu_baseline=False)
         torch.cuda.empty_cache()
         # NOT the headline: the same C2 solve with the residual model compiled
         # into the linearisation kernel (J and f never touch HBM) -- what the
         # solver does when the callback is fusable (VERDICT r1, item 10)
-        inl = run_batched(args, w, "c2", max(2, args.steps // 2), 2, w["B"],
+        inl = run_batched(args, w, "c2", args.steps, args.warmup, w["B"],
                           cpu_baseline=False, inlined=True)
         if rank == 0:
             line["tall"] = tall_line
@@ -762,7 +831,7 @@ def main():
                 "note": "separate record, not the headline: ExpDecay2 compiled into "
                         "the linearisation kernel (models.callbacks(..., 'inlined')); "
                         "results bit-identical to the callback path",
-                "value": inl["value"], "unit": inl["unit"],
+                "value": inl["value"], "unit": inl["unit"], "steps": inl["steps"],
                 "ms_per_step": inl["ms_per_step"], "e2e": inl["e2e"],
                 "step_frac": inl["roofline"]["step_frac"],
                 "gpu_launches": inl["gpu_launches"], "config": inl["config"]}
@@ -780,10 +849,12 @@ def main():
         dist.destroy_process_group()
 
 
-def run_batched(args, w, wname, steps, warmup, B, cpu_baseline=True, inlined=False):
+def run_batched(args, w, wname, steps, warmup, B, cpu_baseline=True, inlined=False,
+                dump_prefix=None):
     """One batched workload on this rank's GPU (problems split by index over
     the ranks, no collective on the data path); returns the JSON record on
-    rank 0, None elsewhere."""
+    rank 0, None elsewhere.  dump_prefix: with --dump-outputs, the last timed
+    step's results go to DIR/<prefix>*.npy."""
     import torch
     import torch.distributed as dist
     from bounded_lsq_b200 import least_squares_batched, PerProblem
@@ -897,6 +968,8 @@ def run_batched(args, w, wname, steps, warmup, B, cpu_baseline=True, inlined=Fal
         e1.record()
         barrier()
     dev_ms = reduce_max(e0.elapsed_time(e1))
+    if args.dump_outputs and dump_prefix is not None and rank == 0:
+        dump_batched(args.dump_outputs, dump_prefix, outs, chunk, B)
     per_step_ms = [a.elapsed_time(b) for a, b in zip(marks, marks[1:])]
     by_rank = None
     if world > 1:

@@ -13,6 +13,7 @@ import numpy as np
 import pytest
 import torch
 
+import packed_npz
 from bounded_lsq_b200 import least_squares, least_squares_batched, PerProblem
 from bounded_lsq_b200.synthetic import ExpDecay2, GaussPeak, RatPoly5
 
@@ -35,7 +36,7 @@ def bits(a, b):
 def check_helpers_bit_exact(lib, dev):
     """bounds.py / dogbox.py:9-35 / FD steps against the reference's outputs
     (tests/golden/helpers.npz), bit for bit."""
-    z = np.load(os.path.join(GOLDEN, "helpers.npz"))
+    z = packed_npz.Packed(os.path.join(GOLDEN, "helpers.npz"))
     n_cases = int(z["ncases"])
     for i in range(n_cases):
         g = lambda k: z[f"c{i}_{k}"]            # noqa: E731

@@ -39,6 +39,7 @@ rt = sys.modules["bounded_lsq.trf"]
 rtr = importlib.import_module("bounded_lsq.trust_region")
 from scipy.optimize._numdiff import approx_derivative  # noqa: E402
 
+import packed_npz                          # noqa: E402
 from oracle import blsq_oracle as orc      # noqa: E402
 from problems import corpus                # noqa: E402
 from bounded_lsq_b200.synthetic import ExpDecay2, GaussPeak, RatPoly5, TallLinExp  # noqa: E402
@@ -231,7 +232,7 @@ def gen_helpers(rng):
     out["meta"] = np.array(json.dumps(dict(
         source="reference bounds.py/dogbox.py + scipy _numdiff",
         oracle_bitwise_equal=True)))
-    np.savez_compressed(os.path.join(HERE, "helpers.npz"), **out)
+    packed_npz.save(os.path.join(HERE, "helpers.npz"), out)
     print("helpers.npz:", len(cases), "cases; oracle bitwise equal")
 
 
@@ -330,7 +331,7 @@ def gen_tr_subproblem(rng):
     out["meta"] = np.array(json.dumps(dict(
         source="reference trust_region.py / trf.py / dogbox.py",
         oracle_bitwise_equal=bool(bit_ok))))
-    np.savez_compressed(os.path.join(HERE, "tr_subproblem.npz"), **out)
+    packed_npz.save(os.path.join(HERE, "tr_subproblem.npz"), out)
     print("tr_subproblem.npz: oracle bitwise equal =", bit_ok)
 
 

@@ -7,6 +7,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -65,8 +66,31 @@ def test_reference_arm_line():
 
 
 @pytest.mark.gpu
-def test_gpu_arm_line():
-    line = run_bench(["--steps", "2", "--warmup", "3", "--no-tall"], 900)
+def test_gpu_arm_line(tmp_path):
+    line = run_bench(["--steps", "2", "--warmup", "3", "--no-tall",
+                      "--dump-outputs", str(tmp_path)], 900)
     check_line(line, reference=False)
+    assert line["steps"] == 2 and len(line["config"]["per_step_ms"]) == 2
     p = line["cpu_baseline"]["parity_vs_gpu"]
     assert p["status_equal"] == 1.0 and p["x_rel_max"] < 1e-8 and p["obj_rel_max"] < 1e-8
+    # --dump-outputs: the last timed step's results on a seeded problem sample
+    files = sorted(os.listdir(tmp_path))
+    assert sum(os.path.getsize(tmp_path / f) for f in files) <= 64 << 20
+    out = {f[:-len(".npy")]: np.load(tmp_path / f) for f in files}
+    assert all(a.dtype == np.float64 for a in out.values())
+    idx = out["problem_index"]
+    assert len(idx) == 32768 and (np.diff(idx) > 0).all()
+    assert out["x"].shape == out["active_mask"].shape == (len(idx), 4)
+    assert out["fun"].shape == (len(idx), 64)
+    assert (out["status"] >= 0).all() and (out["status"] > 0).mean() > 0.99
+    assert np.isfinite(out["obj_value"]).all()
+
+
+@pytest.mark.gpu
+def test_steps_set_every_record():
+    """--steps K times K steps in every record of the default run, the
+    attached tall, c3 and inlined-model records included."""
+    line = run_bench(["--steps", "3", "--warmup", "1", "--no-cpu-baseline"], 900)
+    for rec in (line, line["c3"], line["c2_inlined_model"]):
+        assert rec["steps"] == 3 and len(rec["config"]["per_step_ms"]) == 3
+    assert line["tall"]["steps"] == line["tall_asymmetric_start"]["steps"] == 3

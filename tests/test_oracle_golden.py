@@ -11,6 +11,7 @@ import os
 import numpy as np
 import pytest
 
+import packed_npz
 from oracle import blsq_oracle as orc
 from problems import corpus
 from bounded_lsq_b200.synthetic import ExpDecay2, GaussPeak, TallLinExp
@@ -32,7 +33,7 @@ def _close(a, b, rtol=1e-12):
 
 
 def test_helpers_bit_exact(golden_dir):
-    z = _load(golden_dir, "helpers.npz")
+    z = packed_npz.Packed(os.path.join(golden_dir, "helpers.npz"))
     assert json.loads(str(z["meta"]))["oracle_bitwise_equal"]
     for i in range(int(z["ncases"])):
         g = lambda k: z[f"c{i}_{k}"]            # noqa: E731
@@ -56,7 +57,7 @@ def test_helpers_bit_exact(golden_dir):
 
 
 def test_tr_subproblem(golden_dir):
-    z = _load(golden_dir, "tr_subproblem.npz")
+    z = packed_npz.Packed(os.path.join(golden_dir, "tr_subproblem.npz"))
     for k in range(int(z["n_tr"])):
         g = lambda f: z[f"tr{k}_{f}"]           # noqa: E731
         a0 = float(g("alpha0"))
