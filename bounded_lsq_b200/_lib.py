@@ -39,9 +39,13 @@ SIGNATURES = {
     "blsq_linearise_batched": [_l, _p, _i, _i, _p, _p, _p, _p, _i, _p, _p, _p],
     "blsq_round_batched": [_i, _l, _p, _i, _i, _p, _p, _p, _p, _i, _p,
                            _d, _d, _d, _i, _i, _p, _p, _p, _p, _p, _p, _p],
+    "blsq_linearise_batched_rows": [_l, _p, _i, _i, _p, _p, _p, _p, _i, _p, _p, _p, _p],
+    "blsq_round_batched_rows": [_i, _l, _p, _i, _i, _p, _p, _p, _p, _i, _p,
+                                _d, _d, _d, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p],
     "blsq_dogbox_on_bound": [_l, _i, _p, _p, _p],
     "blsq_count_running": [_l, _p, _p, _p, _p],
     "blsq_model_expdecay2": [_l, _p, _i, _p, _p, _p, _p, _p, _p],
+    "blsq_model_expdecay2_rows": [_l, _p, _i, _p, _p, _p, _p, _p, _p, _p],
     "blsq_model_gausspeak": [_l, _p, _i, _p, _p, _p, _p, _p],
     "blsq_model_expdecay2_linearise": [_l, _p, _i, _p, _p, _p, _p, _p, _p],
     "blsq_model_linexp_fun": [_l, _i, _p, _p, _p, _p, _p, _p],

@@ -172,12 +172,15 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
                   max_nfev, scaling, diff_step=None, check_every=2,
                   compact_below=0.75, tail_below=8192, trace=None,
                   timers=None, graph_tail_rounds=None, prologue=None,
-                  prologue_rounds=6, x_covariance=False, lookahead=None):
+                  prologue_rounds=6, x_covariance=False, lookahead=None, rows=None):
     """Run ``method`` ('trf' | 'dogbox') on B problems.
 
     fun(X, idx) -> (A, m); jac is a callable jac(X, idx) -> (A, m, n) or the
     string '2-point'.  X0 (B, n); lb/ub (n,) or (B, n); scaling (n,) tensor or
-    'jac'.  Returns a dict of device tensors (see least_squares_batched).
+    'jac'.  rows: None, or an int32 (B,) tensor on X0's device -- problem b
+    has residuals 0 .. rows[b]-1 of the (A, m) callback outputs (ragged batch,
+    blsq_linearise_batched_rows / blsq_round_batched_rows).  Returns a dict
+    of device tensors (see least_squares_batched).
     """
     meth = {"trf": L.METHOD_TRF, "dogbox": L.METHOD_DOGBOX}[method]
     dev = X0.device
@@ -203,6 +206,12 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
     fd3 = fd and jac == '3-point'
     npts = 2 * n if fd3 else n                       # callback calls per FD Jacobian
     rel = float("nan") if diff_step is None else float(diff_step)
+    rows_max = None
+    if rows is not None:
+        lib.check_tensor(rows, torch.int32, "rows")
+        if rows.shape != (B,):
+            raise ValueError("`rows` must have shape (B,).")
+        rows_max = int(rows.max().item()) if B else 0
 
     state = torch.zeros((B, S), dtype=f64, device=dev)
     istate = torch.zeros((B, L.ISTATE_SIZE), dtype=torch.int32, device=dev)
@@ -260,6 +269,20 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
     rounds = 0
     launches = 0
 
+    # the dense entry points unless the batch is ragged (same kernels as
+    # before for a dense batch, bit for bit)
+    def lin_call(*a):
+        if rows is None:
+            lib.call("blsq_linearise_batched", *a[:-2], a[-1])
+        else:
+            lib.call("blsq_linearise_batched_rows", *a)
+
+    def round_call(*a):
+        if rows is None:
+            lib.call("blsq_round_batched", *a[:-2], a[-1])
+        else:
+            lib.call("blsq_round_batched_rows", *a)
+
     def one_round(A, idx, idx32, first, nrun, off=0, count_here=True):
         """Callbacks + linearise + round for the A compacted slots (or, in the
         streaming prologue, for the A problems starting at problem `off`)."""
@@ -278,12 +301,14 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
         p_ub = ub.data_ptr() + off * bstride * 8
         p_xn = Xnew.data_ptr() + off * n * 8
         p_xj = None if Xjac is None else Xjac.data_ptr() + off * n * 8
+        # rows is indexed by problem id like istate: shifted the same way
+        p_rows = None if rows is None else rows.data_ptr() + off * 4
         ip = None if idx32 is None else idx32.data_ptr()
         # a model compiled into the linearisation kernel replaces the two
         # callbacks and blsq_linearise_batched of this round by one launch
         cbs = getattr(fun, "__self__", None)
         mm = None
-        if not fd and Xjac is None and hasattr(cbs, "lin"):
+        if not fd and Xjac is None and rows is None and hasattr(cbs, "lin"):
             t0 = tick()
             mm = cbs.lin(Xa, idx32, off, A, p_ist, p_lin, stream)
             if mm is not None:
@@ -299,6 +324,9 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
             F = F.contiguous()
             if m is None:
                 m = F.shape[1]
+                if rows_max is not None and rows_max > m:
+                    raise ValueError(f"`rows` exceeds the {m} residuals `fun` returns "
+                                     f"(max(rows) = {rows_max}).")
             elif F.shape[1] != m:
                 raise RuntimeError("`fun` changed its number of residuals")
             if not fd:
@@ -313,8 +341,8 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
                 J = J.contiguous()
                 tock("callbacks", t0, nrun)
                 t0 = tick()
-                lib.call("blsq_linearise_batched", A, ip, m, n, F.data_ptr(),
-                         J.data_ptr(), None, None, 0, p_ist, p_lin, stream)
+                lin_call(A, ip, m, n, F.data_ptr(), J.data_ptr(), None, None, 0,
+                         p_ist, p_lin, p_rows, stream)
                 tock("linearise", t0, nrun)
             else:
                 Xpa = Xp.view(-1)[: npts * A * n].view(npts, A, n)
@@ -331,17 +359,17 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
                 plist = (C.c_void_p * npts)(*[t.data_ptr() for t in Fp])
                 tock("callbacks", t0, nrun)
                 t0 = tick()
-                lib.call("blsq_linearise_batched", A, ip, m, n, F.data_ptr(), None,
+                lin_call(A, ip, m, n, F.data_ptr(), None,
                          C.cast(plist, C.c_void_p), dx.data_ptr(), 2 if fd3 else 1,
-                         p_ist, p_lin, stream)
+                         p_ist, p_lin, p_rows, stream)
                 tock("linearise", t0, nrun)
         t0 = tick()
-        lib.call("blsq_round_batched", meth, A, ip, m, n, p_lin,
-                 p_x0, p_lb, p_ub, bstride, sc_ptr,
-                 float(ftol), float(xtol), float(gtol), max_nfev, first,
-                 p_st, p_ist, p_xn, p_xj,
-                 rwork_ptr if A >= TWO_KERNELS_ABOVE else None,
-                 count.data_ptr() if (count_here and fused_count) else None, stream)
+        round_call(meth, A, ip, m, n, p_lin,
+                   p_x0, p_lb, p_ub, bstride, sc_ptr,
+                   float(ftol), float(xtol), float(gtol), max_nfev, first,
+                   p_st, p_ist, p_xn, p_xj,
+                   rwork_ptr if A >= TWO_KERNELS_ABOVE else None,
+                   count.data_ptr() if (count_here and fused_count) else None, p_rows, stream)
         tock("round", t0, nrun)
         if timers is not None:
             timers["shape"] = (n, m, LS, S)

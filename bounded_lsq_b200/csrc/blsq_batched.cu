@@ -58,7 +58,7 @@ namespace {
 #define BLSQ_PREFETCH(p) asm volatile("prefetch.global.L2 [%0];" ::"l"(p))
 #endif
 
-template <int N, int METHOD, int MODE>
+template <int N, int METHOD, int MODE, bool ROWS>
 __device__ __forceinline__ bool
 round_slot(int64_t slot, int64_t A, const int32_t* __restrict__ idx,
            const double* __restrict__ lin, const double* __restrict__ x0,
@@ -66,13 +66,23 @@ round_slot(int64_t slot, int64_t A, const int32_t* __restrict__ idx,
            int bstride, const double* __restrict__ scaling, const SolveParams& P,
            int first, double* __restrict__ state,
            int32_t* __restrict__ istate, double* __restrict__ Xnew,
-           double* __restrict__ Xjac, int32_t* __restrict__ work) {
+           double* __restrict__ Xjac, int32_t* __restrict__ work,
+           const int32_t* __restrict__ rows) {
     typedef LinRec<N> L;
     constexpr int SS = (METHOD == BLSQ_METHOD_TRF) ? TrfState<N>::SIZE
                                                    : DogState<N>::SIZE;
     if (slot >= A) return false;
     const int64_t pid = idx ? idx[slot] : slot;
     int32_t* ip = istate + pid * IS_SIZE;
+    // ROWS, a ragged batch: the decisions that use m (full_rank, the
+    // Gauss-Newton certificate, dogbox's rcond) see this problem's own number
+    // of rows.  A separate instance: a runtime test here costs the dense
+    // TRF rounds spill traffic.
+    SolveParams Pp = P;
+    if (ROWS) {
+        const int r = rows[pid];
+        Pp.m = r < 0 ? 0 : (r > P.m ? P.m : r);
+    }
     double sc[N];
 #pragma unroll
     for (int i = 0; i < N; i++) sc[i] = scaling ? scaling[i] : 1.0;
@@ -104,7 +114,7 @@ round_slot(int64_t slot, int64_t A, const int32_t* __restrict__ idx,
         if (ist[IS_STATUS] != ST_RUNNING) return false;
         const int rc = trf_round_impl<N, MODE>(
             state + pid * (int64_t)SS, ist, lin + slot * (int64_t)L::SIZE, x0 + pid * N,
-            lb + pid * bstride, ub + pid * bstride, sc, P, first, Xnew + slot * N);
+            lb + pid * bstride, ub + pid * bstride, sc, Pp, first, Xnew + slot * N);
         *reinterpret_cast<int4*>(ip) = make_int4(ist[0], ist[1], ist[2], ist[3]);
         if (MODE == 1 && rc == TRF_DEFER)
             work[1 + atomicAdd(work, 1)] = (int32_t)slot;
@@ -143,7 +153,7 @@ round_slot(int64_t slot, int64_t A, const int32_t* __restrict__ idx,
         }
     }
     const bool go = dogbox_round<N>(st, ist, ln, x0 + pid * N, lb + pid * bstride,
-                                    ub + pid * bstride, sc, P, first);
+                                    ub + pid * bstride, sc, Pp, first);
     if (SS % 2 == 0) {
 #pragma unroll
         for (int i = 0; i < SS; i += 2)
@@ -183,7 +193,7 @@ template <int N, int METHOD> struct RoundCfg {
                                                 : BLSQ_ROUND_MINB;
 };
 
-template <int N, int METHOD, int MODE>
+template <int N, int METHOD, int MODE, bool ROWS>
 __global__ void __launch_bounds__(BLSQ_ROUND_THREADS, (RoundCfg<N, METHOD>::MINB))
 round_kernel(int64_t A, const int32_t* __restrict__ idx,
              const double* __restrict__ lin, const double* __restrict__ x0,
@@ -192,19 +202,19 @@ round_kernel(int64_t A, const int32_t* __restrict__ idx,
              int first, double* __restrict__ state,
              int32_t* __restrict__ istate, double* __restrict__ Xnew,
              double* __restrict__ Xjac, int32_t* __restrict__ work,
-             int32_t* __restrict__ count) {
+             int32_t* __restrict__ count, const int32_t* __restrict__ rows) {
     const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (MODE == 2) {
         // the worklist length is only known on the device: a small grid
         // strides over it
         const int64_t cnt = work[0];
         for (int64_t w = tid; w < cnt; w += (int64_t)gridDim.x * blockDim.x)
-            round_slot<N, METHOD, MODE>(work[1 + w], A, idx, lin, x0, lb, ub, bstride, scaling,
-                                        P, first, state, istate, Xnew, Xjac, work);
+            round_slot<N, METHOD, MODE, ROWS>(work[1 + w], A, idx, lin, x0, lb, ub, bstride, scaling,
+                                        P, first, state, istate, Xnew, Xjac, work, rows);
         return;
     }
-    const bool run = round_slot<N, METHOD, MODE>(tid, A, idx, lin, x0, lb, ub, bstride, scaling,
-                                                 P, first, state, istate, Xnew, Xjac, work);
+    const bool run = round_slot<N, METHOD, MODE, ROWS>(tid, A, idx, lin, x0, lb, ub, bstride, scaling,
+                                                 P, first, state, istate, Xnew, Xjac, work, rows);
     if (!count) return;
     // running problems after this round: one atomic per CTA; the last CTA to
     // arrive publishes the total in count[2] and re-arms the two counters, so
@@ -380,79 +390,107 @@ compact_scatter_kernel(int64_t A, const int32_t* __restrict__ idx,
     }
 }
 
+template <int N, int G, bool MULTI, bool ROWS>
+int launch_lin_r(unsigned blocks, int64_t A, const int32_t* idx, int m, const double* F,
+                 const double* J, const PtrList<N>& pl, const double* dx,
+                 int jac_mode, const int32_t* istate, double* lin,
+                 const int32_t* rows, cudaStream_t s) {
+    if (jac_mode == 0)
+        lin_kernel<N, G, 0, MULTI, NoModel, ROWS><<<blocks, BLSQ_LIN_THREADS, 0, s>>>(
+            A, idx, m, F, J, pl, dx, istate, lin, NoModel(), rows);
+    else if (jac_mode == 1)
+        lin_kernel<N, G, 1, MULTI, NoModel, ROWS><<<blocks, BLSQ_LIN_THREADS, 0, s>>>(
+            A, idx, m, F, J, pl, dx, istate, lin, NoModel(), rows);
+    else
+        lin_kernel<N, G, 2, MULTI, NoModel, ROWS><<<blocks, BLSQ_LIN_THREADS, 0, s>>>(
+            A, idx, m, F, J, pl, dx, istate, lin, NoModel(), rows);
+    BLSQ_LAUNCH_CHECK();
+    return 0;
+}
+
+// rows == null: the dense instances; else the ragged ones (lin_kernel ROWS)
 template <int N, int G, bool MULTI>
 int launch_lin_g(int64_t A, const int32_t* idx, int m, const double* F,
                  const double* J, const PtrList<N>& pl, const double* dx,
                  int jac_mode, const int32_t* istate, double* lin,
-                 cudaStream_t s) {
+                 const int32_t* rows, cudaStream_t s) {
     int64_t threads = A * G;
     int64_t blocks = (threads + BLSQ_LIN_THREADS - 1) / BLSQ_LIN_THREADS;
     if (blocks > 0x7fffffff) return BLSQ_E_UNSUPPORTED;
-    if (jac_mode == 0)
-        lin_kernel<N, G, 0, MULTI><<<(unsigned)blocks, BLSQ_LIN_THREADS, 0, s>>>(
-            A, idx, m, F, J, pl, dx, istate, lin);
-    else if (jac_mode == 1)
-        lin_kernel<N, G, 1, MULTI><<<(unsigned)blocks, BLSQ_LIN_THREADS, 0, s>>>(
-            A, idx, m, F, J, pl, dx, istate, lin);
-    else
-        lin_kernel<N, G, 2, MULTI><<<(unsigned)blocks, BLSQ_LIN_THREADS, 0, s>>>(
-            A, idx, m, F, J, pl, dx, istate, lin);
-    BLSQ_LAUNCH_CHECK();
-    return 0;
+    if (rows)
+        return launch_lin_r<N, G, MULTI, true>((unsigned)blocks, A, idx, m, F, J, pl, dx,
+                                               jac_mode, istate, lin, rows, s);
+    return launch_lin_r<N, G, MULTI, false>((unsigned)blocks, A, idx, m, F, J, pl, dx,
+                                            jac_mode, istate, lin, nullptr, s);
 }
 
 template <int N>
 int launch_lin(int64_t A, const int32_t* idx, int m, const double* F,
                const double* J, const double* const* Fp_host, const double* dx,
                int jac_mode, const int32_t* istate, double* lin,
-               cudaStream_t s) {
+               const int32_t* rows, cudaStream_t s) {
     constexpr int RPL = LinCfg<N>::RPL;
     PtrList<N> pl;
     const int np = jac_mode == 2 ? 2 * N : (jac_mode == 1 ? N : 0);
     for (int j = 0; j < 2 * N; j++) pl.p[j] = (j < np) ? Fp_host[j] : nullptr;
-    // smallest lane group whose registers hold all m rows (else 32 + chunks)
+    // smallest lane group whose registers hold all m rows (else 32 + chunks);
+    // a ragged batch is classed by its width m, not by its counts
     if (m <= 8 * RPL)
-        return launch_lin_g<N, 8, false>(A, idx, m, F, J, pl, dx, jac_mode, istate, lin, s);
+        return launch_lin_g<N, 8, false>(A, idx, m, F, J, pl, dx, jac_mode, istate, lin, rows, s);
     if (m <= 16 * RPL)
-        return launch_lin_g<N, 16, false>(A, idx, m, F, J, pl, dx, jac_mode, istate, lin, s);
+        return launch_lin_g<N, 16, false>(A, idx, m, F, J, pl, dx, jac_mode, istate, lin, rows, s);
     if (m <= 32 * RPL)
-        return launch_lin_g<N, 32, false>(A, idx, m, F, J, pl, dx, jac_mode, istate, lin, s);
-    return launch_lin_g<N, 32, true>(A, idx, m, F, J, pl, dx, jac_mode, istate, lin, s);
+        return launch_lin_g<N, 32, false>(A, idx, m, F, J, pl, dx, jac_mode, istate, lin, rows, s);
+    return launch_lin_g<N, 32, true>(A, idx, m, F, J, pl, dx, jac_mode, istate, lin, rows, s);
 }
 
-template <int N>
-int launch_round(int method, int64_t A, const int32_t* idx, const double* lin,
+template <int N, bool ROWS>
+int launch_round_r(int method, int64_t A, const int32_t* idx, const double* lin,
                  const double* x0, const double* lb, const double* ub,
                  int bstride, const double* scaling, SolveParams P, int first,
                  double* state, int32_t* istate, double* Xnew, double* Xjac,
-                 int32_t* work, int32_t* count, cudaStream_t s) {
+                 int32_t* work, int32_t* count, const int32_t* rows, cudaStream_t s) {
     int64_t blocks = (A + BLSQ_ROUND_THREADS - 1) / BLSQ_ROUND_THREADS;
     if (blocks > 0x7fffffff) return BLSQ_E_UNSUPPORTED;
     const unsigned gb = (unsigned)blocks;
     if (method == BLSQ_METHOD_TRF && work) {
         cudaError_t e = cudaMemsetAsync(work, 0, sizeof(int32_t), s);
         if (e != cudaSuccess) return (int)e;
-        round_kernel<N, BLSQ_METHOD_TRF, 1><<<gb, BLSQ_ROUND_THREADS, 0, s>>>(
+        round_kernel<N, BLSQ_METHOD_TRF, 1, ROWS><<<gb, BLSQ_ROUND_THREADS, 0, s>>>(
             A, idx, lin, x0, lb, ub, bstride, scaling, P, first, state, istate, Xnew, Xjac, work,
-            count);
+            count, rows);
         BLSQ_LAUNCH_CHECK();
         // ~5 % of the problems land on the worklist: an eighth of the grid
         // (at least 4 CTAs per SM) strides over it
         unsigned g2 = gb / 8 > 592u ? gb / 8 : (gb < 592u ? gb : 592u);
-        round_kernel<N, BLSQ_METHOD_TRF, 2><<<g2, BLSQ_ROUND_THREADS, 0, s>>>(
+        round_kernel<N, BLSQ_METHOD_TRF, 2, ROWS><<<g2, BLSQ_ROUND_THREADS, 0, s>>>(
             A, idx, lin, x0, lb, ub, bstride, scaling, P, first, state, istate, Xnew, Xjac, work,
-            nullptr);
+            nullptr, rows);
     } else if (method == BLSQ_METHOD_TRF) {
-        round_kernel<N, BLSQ_METHOD_TRF, 0><<<gb, BLSQ_ROUND_THREADS, 0, s>>>(
+        round_kernel<N, BLSQ_METHOD_TRF, 0, ROWS><<<gb, BLSQ_ROUND_THREADS, 0, s>>>(
             A, idx, lin, x0, lb, ub, bstride, scaling, P, first, state, istate, Xnew, Xjac, work,
-            count);
+            count, rows);
     } else {
-        round_kernel<N, BLSQ_METHOD_DOGBOX, 0><<<gb, BLSQ_ROUND_THREADS, 0, s>>>(
+        round_kernel<N, BLSQ_METHOD_DOGBOX, 0, ROWS><<<gb, BLSQ_ROUND_THREADS, 0, s>>>(
             A, idx, lin, x0, lb, ub, bstride, scaling, P, first, state, istate, Xnew, Xjac, work,
-            count);
+            count, rows);
     }
     BLSQ_LAUNCH_CHECK();
     return 0;
+}
+
+// rows == null: the dense instances; else the ragged ones (round_slot ROWS)
+template <int N>
+int launch_round(int method, int64_t A, const int32_t* idx, const double* lin,
+                 const double* x0, const double* lb, const double* ub,
+                 int bstride, const double* scaling, SolveParams P, int first,
+                 double* state, int32_t* istate, double* Xnew, double* Xjac,
+                 int32_t* work, int32_t* count, const int32_t* rows, cudaStream_t s) {
+    if (rows)
+        return launch_round_r<N, true>(method, A, idx, lin, x0, lb, ub, bstride, scaling, P,
+                                       first, state, istate, Xnew, Xjac, work, count, rows, s);
+    return launch_round_r<N, false>(method, A, idx, lin, x0, lb, ub, bstride, scaling, P,
+                                    first, state, istate, Xnew, Xjac, work, count, nullptr, s);
 }
 
 }  // namespace
@@ -522,11 +560,11 @@ int blsq_init_batched(int method, int64_t B, int n, const double* x0,
     return 0;
 }
 
-int blsq_linearise_batched(int64_t A, const int32_t* idx, int m, int n,
-                           const double* F, const double* J,
-                           const double* const* Fp_host, const double* dx,
-                           int jac_mode, const int32_t* istate, double* lin,
-                           void* stream) {
+int blsq_linearise_batched_rows(int64_t A, const int32_t* idx, int m, int n,
+                                const double* F, const double* J,
+                                const double* const* Fp_host, const double* dx,
+                                int jac_mode, const int32_t* istate, double* lin,
+                                const int32_t* rows, void* stream) {
     if (A < 0 || m < 1 || !F || !istate || !lin) return BLSQ_E_BADARG;
     if (jac_mode < 0 || jac_mode > 2) return BLSQ_E_BADARG;
     if (jac_mode == 0 && !J) return BLSQ_E_BADARG;
@@ -537,17 +575,27 @@ int blsq_linearise_batched(int64_t A, const int32_t* idx, int m, int n,
     if (A == 0) return 0;
     BLSQ_DISPATCH_N(n, {
         return launch_lin<N_>(A, idx, m, F, J, Fp_host, dx, jac_mode, istate,
-                              lin, (cudaStream_t)stream);
+                              lin, rows, (cudaStream_t)stream);
     });
     return 0;
 }
 
-int blsq_round_batched(int method, int64_t A, const int32_t* idx, int m, int n,
-                       const double* lin, const double* x0, const double* lb,
-                       const double* ub, int bstride, const double* scaling,
-                       double ftol, double xtol, double gtol, int max_nfev,
-                       int first, double* state, int32_t* istate, double* Xnew,
-                       double* Xjac, int32_t* work, int32_t* count, void* stream) {
+int blsq_linearise_batched(int64_t A, const int32_t* idx, int m, int n,
+                           const double* F, const double* J,
+                           const double* const* Fp_host, const double* dx,
+                           int jac_mode, const int32_t* istate, double* lin,
+                           void* stream) {
+    return blsq_linearise_batched_rows(A, idx, m, n, F, J, Fp_host, dx, jac_mode, istate,
+                                       lin, nullptr, stream);
+}
+
+int blsq_round_batched_rows(int method, int64_t A, const int32_t* idx, int m, int n,
+                            const double* lin, const double* x0, const double* lb,
+                            const double* ub, int bstride, const double* scaling,
+                            double ftol, double xtol, double gtol, int max_nfev,
+                            int first, double* state, int32_t* istate, double* Xnew,
+                            double* Xjac, int32_t* work, int32_t* count,
+                            const int32_t* rows, void* stream) {
     if (A < 0 || !lin || !x0 || !lb || !ub || !state || !istate || !Xnew) return BLSQ_E_BADARG;
     if (method != BLSQ_METHOD_TRF && method != BLSQ_METHOD_DOGBOX) return BLSQ_E_BADARG;
     if (bstride != 0 && bstride != n) return BLSQ_E_BADARG;
@@ -564,9 +612,20 @@ int blsq_round_batched(int method, int64_t A, const int32_t* idx, int m, int n,
     BLSQ_DISPATCH_N(n, {
         return launch_round<N_>(method, A, idx, lin, x0, lb, ub, bstride,
                                 scaling, P, first, state, istate, Xnew, Xjac,
-                                work, count, (cudaStream_t)stream);
+                                work, count, rows, (cudaStream_t)stream);
     });
     return 0;
+}
+
+int blsq_round_batched(int method, int64_t A, const int32_t* idx, int m, int n,
+                       const double* lin, const double* x0, const double* lb,
+                       const double* ub, int bstride, const double* scaling,
+                       double ftol, double xtol, double gtol, int max_nfev,
+                       int first, double* state, int32_t* istate, double* Xnew,
+                       double* Xjac, int32_t* work, int32_t* count, void* stream) {
+    return blsq_round_batched_rows(method, A, idx, m, n, lin, x0, lb, ub, bstride, scaling,
+                                   ftol, xtol, gtol, max_nfev, first, state, istate, Xnew,
+                                   Xjac, work, count, nullptr, stream);
 }
 
 int blsq_dogbox_on_bound(int64_t B, int n, const int32_t* istate,

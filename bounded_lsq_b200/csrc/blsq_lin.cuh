@@ -92,13 +92,20 @@ template <int N> struct PtrList { const double* p[2 * N]; };   // 2 per coordina
 // triangle carried in one extra register row; otherwise all rows are resident,
 // g / f.f are reduced and written before the sweep and row k of the triangle
 // is stored by lane k as soon as it exists (fewer live registers).
-template <int N, int G, int MODE, bool MULTI, class MODEL = NoModel>
+// ROWS: ragged batch, problem pid has rows[pid] (clamped to [0, m]) residuals
+// and m is only the row stride of F / J / Fpert.  Rows past the count are
+// never read and enter the sweep as zeros, exactly like the rows past m of a
+// partial last chunk, so a ragged problem gets the record of a dense solve of
+// its first rows[pid] residuals with the same lane group.  MULTI folds chunks
+// only up to the problem's own count.  The dense path (ROWS = false) is a
+// separate instance and compiles to the code it had before.
+template <int N, int G, int MODE, bool MULTI, class MODEL = NoModel, bool ROWS = false>
 __global__ void __launch_bounds__(BLSQ_LIN_THREADS, LinCfg<N>::MINB)
 lin_kernel(int64_t A, const int32_t* __restrict__ idx, int m,
            const double* __restrict__ F, const double* __restrict__ J,
            PtrList<N> Fpert, const double* __restrict__ dx,
            const int32_t* __restrict__ istate, double* __restrict__ lin,
-           MODEL mdl = MODEL()) {
+           MODEL mdl = MODEL(), const int32_t* __restrict__ rows = nullptr) {
     constexpr int RPL = LinCfg<N>::RPL;
     constexpr int C = N + 1;                      // columns of [J | f]
     constexpr int AR = MULTI ? RPL + 1 : RPL;     // + carried row of the triangle
@@ -114,6 +121,12 @@ lin_kernel(int64_t A, const int32_t* __restrict__ idx, int m,
     }
     if (!__any_sync(0xffffffffu, valid)) return;
     const bool all_valid = __all_sync(0xffffffffu, valid);
+    // rows of this problem (ROWS; MULTI: G = 32, so the count is warp-uniform)
+    int mp = m;
+    if (ROWS && valid) {
+        const int r = rows[pid];
+        mp = r < 0 ? 0 : (r > m ? m : r);
+    }
 
     const double* Fp = (MODE == 3) ? nullptr : F + slot * (int64_t)m;
     const double* Jp = (MODE == 0) ? J + slot * (int64_t)m * N : nullptr;
@@ -129,8 +142,10 @@ lin_kernel(int64_t A, const int32_t* __restrict__ idx, int m,
         for (int j = 0; j < C; j++) { myrow[j] = 0.0; a[AR - 1][j] = 0.0; }
     }
 
-    for (int base = 0; base < (MULTI ? m : 1); base += G * RPL) {
-        const bool full = all_valid && (base + G * RPL <= m);   // warp-uniform
+    for (int base = 0; base < (MULTI ? mp : 1); base += G * RPL) {
+        // warp-uniform: every group of the warp loads the whole chunk
+        const bool full = ROWS ? __all_sync(0xffffffffu, valid && base + G * RPL <= mp)
+                               : all_valid && (base + G * RPL <= m);
         // ---- load this chunk ----
         {
             double dxj[N], dxr[N];
@@ -153,7 +168,7 @@ lin_kernel(int64_t A, const int32_t* __restrict__ idx, int m,
 #pragma unroll
             for (int s = 0; s < RPL; s++) {
                 int row = base + s * G + lane;
-                bool ok = full || (valid && row < m);
+                bool ok = full || (valid && row < mp);
                 if (ok && MODE == 3) {
                     mdl.template row<N>(slot, pid, row, a[s]);
                 } else if (ok) {

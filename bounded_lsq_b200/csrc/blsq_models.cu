@@ -37,17 +37,28 @@ struct ExpDecay2Rows {
 #define BLSQ_EXPDECAY2_QUADS 1
 #endif
 
+// ROWS: ragged batch, problem pid has rows[pid] residuals (clamped to
+// [0, m]); rows past the count are neither read nor written
+template <bool ROWS>
+__device__ __forceinline__ int model_rows(const int32_t* rows, int64_t pid, int m) {
+    if (!ROWS) return m;
+    const int r = rows[pid];
+    return r < 0 ? 0 : (r > m ? m : r);
+}
+
+template <bool ROWS>
 __global__ void __launch_bounds__(256)
 expdecay2_kernel(int64_t A, const int64_t* __restrict__ idx, int m,
                  const double* __restrict__ t, const double* __restrict__ X,
                  const double* __restrict__ y, double* __restrict__ F,
-                 double* __restrict__ J) {
+                 double* __restrict__ J, const int32_t* __restrict__ rows) {
     // block = (rows, problems): no 64-bit division per element
     const int64_t s = (int64_t)blockIdx.x * blockDim.y + threadIdx.y;
     const int r = blockIdx.y * blockDim.x + threadIdx.x;
     if (s >= A || r >= m) return;
     const int64_t g = s * m + r;
     int64_t pid = idx ? idx[s] : s;
+    if (ROWS && r >= model_rows<ROWS>(rows, pid, m)) return;
     const double4 x = *reinterpret_cast<const double4*>(X + s * 4);
     const double tr = t[r];
     // same operation order as synthetic.ExpDecay2.fun_t / jac_t
@@ -66,17 +77,22 @@ expdecay2_kernel(int64_t A, const int64_t* __restrict__ idx, int m,
 }
 
 // m % 4 == 0: one thread per (problem, four consecutive rows): 256-bit loads of
-// t and y, one 256-bit store of F and four of J (128 contiguous bytes)
+// t and y, one 256-bit store of F and four of J (128 contiguous bytes).  ROWS:
+// the quad that straddles the problem's count stores only its rows below it
+// (it reads all four: they lie inside the (A, m) buffers)
+template <bool ROWS>
 __global__ void __launch_bounds__(256)
 expdecay2x4_kernel(int64_t A, const int64_t* __restrict__ idx, int m,
                    const double* __restrict__ t, const double* __restrict__ X,
                    const double* __restrict__ y, double* __restrict__ F,
-                   double* __restrict__ J) {
+                   double* __restrict__ J, const int32_t* __restrict__ rows) {
     const int64_t s = (int64_t)blockIdx.x * blockDim.y + threadIdx.y;
     const int r = 4 * (blockIdx.y * blockDim.x + threadIdx.x);
     if (s >= A || r >= m) return;
     const int64_t g = s * m + r;
     const int64_t pid = idx ? idx[s] : s;
+    const int nk = ROWS ? model_rows<ROWS>(rows, pid, m) - r : 4;   // rows of this quad
+    if (ROWS && nk <= 0) return;
     const double4 x = *reinterpret_cast<const double4*>(X + s * 4);
     double tr[4], yv[4], f[4];
     asm volatile("ld.global.nc.v4.f64 {%0,%1,%2,%3}, [%4];"
@@ -91,12 +107,16 @@ expdecay2x4_kernel(int64_t A, const int64_t* __restrict__ idx, int m,
         const double e1 = exp(-x.y * tr[k]);
         const double e2 = exp(-x.w * tr[k]);
         f[k] = x.x * e1 + x.z * e2 - yv[k];
-        if (J) {
+        if (J && (!ROWS || k < nk)) {
             const double j1 = -x.x * tr[k] * e1, j3 = -x.z * tr[k] * e2;
             asm volatile("st.global.cs.v4.f64 [%0], {%1,%2,%3,%4};" ::"l"(J + (g + k) * 4),
                          "d"(e1), "d"(j1), "d"(e2), "d"(j3)
                          : "memory");
         }
+    }
+    if (ROWS && nk < 4) {
+        for (int k = 0; k < nk; k++) F[g + k] = f[k];
+        return;
     }
     asm volatile("st.global.cs.v4.f64 [%0], {%1,%2,%3,%4};" ::"l"(F + g), "d"(f[0]), "d"(f[1]),
                  "d"(f[2]), "d"(f[3])
@@ -315,21 +335,32 @@ int blsq_model_expdecay2_linearise(int64_t A, const int32_t* idx, int m, const d
     return 0;
 }
 
-int blsq_model_expdecay2(int64_t A, const int64_t* idx, int m, const double* t,
-                         const double* X, const double* y, double* F, double* J,
-                         void* stream) {
+int blsq_model_expdecay2_rows(int64_t A, const int64_t* idx, int m, const double* t,
+                              const double* X, const double* y, const int32_t* rows,
+                              double* F, double* J, void* stream) {
     if (A < 0 || m < 1 || !t || !X || !y || !F) return BLSQ_E_BADARG;
     if (A == 0) return 0;
     dim3 block, grid;
     const bool quads = BLSQ_EXPDECAY2_QUADS && m % 4 == 0 && ((uintptr_t)t % 32 == 0) &&
                        ((uintptr_t)y % 32 == 0) && ((uintptr_t)F % 32 == 0);
     if (!batched_model_grid(A, quads ? m / 4 : m, block, grid)) return BLSQ_E_UNSUPPORTED;
-    if (quads)
-        expdecay2x4_kernel<<<grid, block, 0, (cudaStream_t)stream>>>(A, idx, m, t, X, y, F, J);
+    cudaStream_t s = (cudaStream_t)stream;
+    if (quads && rows)
+        expdecay2x4_kernel<true><<<grid, block, 0, s>>>(A, idx, m, t, X, y, F, J, rows);
+    else if (quads)
+        expdecay2x4_kernel<false><<<grid, block, 0, s>>>(A, idx, m, t, X, y, F, J, nullptr);
+    else if (rows)
+        expdecay2_kernel<true><<<grid, block, 0, s>>>(A, idx, m, t, X, y, F, J, rows);
     else
-        expdecay2_kernel<<<grid, block, 0, (cudaStream_t)stream>>>(A, idx, m, t, X, y, F, J);
+        expdecay2_kernel<false><<<grid, block, 0, s>>>(A, idx, m, t, X, y, F, J, nullptr);
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? 0 : (int)e;
+}
+
+int blsq_model_expdecay2(int64_t A, const int64_t* idx, int m, const double* t,
+                         const double* X, const double* y, double* F, double* J,
+                         void* stream) {
+    return blsq_model_expdecay2_rows(A, idx, m, t, X, y, nullptr, F, J, stream);
 }
 
 int blsq_model_gausspeak(int64_t A, const int64_t* idx, int m, const double* t,

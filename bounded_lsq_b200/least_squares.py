@@ -139,8 +139,21 @@ def least_squares_batched(fun, x0, jac='2-point', bounds=(-float('inf'), float('
     Every field of the result has a leading B dimension.
 
     ``options``: ``chunk`` (solve the batch that many problems at a time),
-    ``x_covariance``, ``h2d_chunks`` / ``device`` (host inputs), and the driver
-    knobs of ``batched.solve_batched``.
+    ``x_covariance``, ``h2d_chunks`` / ``device`` (host inputs), ``rows``
+    (ragged batches, below), and the driver knobs of ``batched.solve_batched``.
+
+    Ragged batches, ``options={'rows': rows}``: ``rows`` is an integer tensor of
+    shape (B,), on the CPU or on the solve's device.  The callbacks keep
+    returning dense (A, m) / (A, m, n) tensors, m being the padded width, but
+    problem b only has residuals 0 .. rows[b]-1: the rows past it are never
+    read and may hold anything, NaN included.  Each problem is solved as the
+    reference solves the problem made of its first rows[b] residuals (cost,
+    full-rank test, Gauss-Newton certificate, dogbox's rcond).  ``res.fun`` is
+    zero past rows[b].  A callback that wants the counts takes them as one more
+    argument, ``args=(..., PerProblem(rows))``: they are gathered and chunked
+    like the other per-problem data.  Not available with models compiled into
+    the linearisation (``models.callbacks(..., 'inlined')``).  Without
+    ``rows`` the solve is exactly the dense one.
     """
     lib = _lib if _lib is not None else L.get_lib()
     _validate_common(method, bounds, jac)
@@ -155,6 +168,9 @@ def least_squares_batched(fun, x0, jac='2-point', bounds=(-float('inf'), float('
     guard = torch.cuda.device(target) if target is not None else \
         lib.device_guard(None)
     chunk = options.pop("chunk", None)
+    if options.get("rows") is not None and getattr(fun, "blsq_linearise", None) is not None:
+        raise ValueError("`rows` is not supported with a model compiled into the "
+                         "linearisation (models.callbacks(..., 'inlined')).")
     with guard:
         if chunk is not None and isinstance(x0, torch.Tensor) and x0.dim() == 2 \
                 and x0.shape[0] > int(chunk) > 0:
@@ -175,11 +191,14 @@ def _least_squares_chunked(lib, chunk, fun, x0, jac, bounds, method, ftol, xtol,
     when its own copies have landed."""
     B = x0.shape[0]
     plan = None
+    rows = options.pop("rows", None)
     if lib.requires_cuda and not x0.is_cuda:
         x0, args, kwargs, plan = _stage_host_inputs(x0, args, kwargs, options)
     else:
         options.pop("h2d_chunks", None)
         options.pop("device", None)
+    if rows is not None:
+        rows = _check_rows(rows, B, x0.device)         # copied once, sliced per chunk
 
     def part(v, c0, c1):
         if isinstance(v, PerProblem):
@@ -201,11 +220,14 @@ def _least_squares_chunked(lib, chunk, fun, x0, jac, bounds, method, ftol, xtol,
             for p0, p1, ev in plan:
                 if ev is not None and p0 < c1 and p1 > c0:
                     cur.wait_event(ev)
+        opts = dict(options)
+        if rows is not None:
+            opts["rows"] = rows[c0:c1]
         outs.append(_least_squares_batched(
             lib, fun, x0[c0:c1], jac, (bound(bounds[0], c0, c1), bound(bounds[1], c0, c1)),
             method, ftol, xtol, gtol, max_nfev, scaling, diff_step,
             tuple(part(v, c0, c1) for v in args),
-            {k: part(v, c0, c1) for k, v in dict(kwargs).items()}, dict(options)))
+            {k: part(v, c0, c1) for k, v in dict(kwargs).items()}, opts))
     res = OptimizeResult(outs[0])
     for key, v in outs[0].items():
         if isinstance(v, torch.Tensor) and v.dim() >= 1 and v.shape[0] == outs[0].x.shape[0]:
@@ -261,13 +283,21 @@ def _least_squares_batched(lib, fun, x0, jac, bounds, method, ftol, xtol, gtol,
     for v in list(args) + list(dict(kwargs).values()):
         if isinstance(v, PerProblem):
             lib.same_device(x0, PerProblem=v.tensor)
+    rows = options.pop("rows", None)
+    if rows is not None:
+        rows = _check_rows(rows, B, x0.device)
 
     cb = BatchedCallbacks(fun, jac, args, kwargs, B)
     jarg = jac if isinstance(jac, str) else cb.j
     out = solve_batched(lib, method, cb.f, jarg, x0, lb, ub, ftol, xtol, gtol,
-                        max_nfev, scaling, diff_step=diff_step, **options)
+                        max_nfev, scaling, diff_step=diff_step, rows=rows, **options)
     res = OptimizeResult(out)
     res.fun = cb.f(res.x, None)
+    if rows is not None:
+        # the padding of a ragged batch is not part of the residual vector
+        m = res.fun.shape[1]
+        pad = torch.arange(m, device=res.fun.device)[None, :] >= rows[:, None].to(res.fun.device)
+        res.fun = res.fun.masked_fill(pad, 0.0)
     release = getattr(fun, "blsq_release", None)
     if callable(release):
         release()                          # callbacks that cache between fun and jac
@@ -278,6 +308,27 @@ def _least_squares_batched(lib, fun, x0, jac, bounds, method, ftol, xtol, gtol,
         "ValueError: `x` is not within the trust region."
     res.success = res.status > 0
     return res
+
+
+def _check_rows(rows, B, dev):
+    """``options['rows']``: an integer tensor of shape (B,) with every count
+    >= 1 (the upper limit m is checked at the first residual evaluation), as
+    a contiguous int32 tensor on ``dev``."""
+    if not isinstance(rows, torch.Tensor):
+        try:
+            rows = torch.as_tensor(rows)
+        except (TypeError, ValueError, RuntimeError):
+            raise ValueError("`rows` must be an integer tensor of shape (B,).")
+    if rows.dtype.is_floating_point or rows.dtype.is_complex or rows.dtype == torch.bool:
+        raise ValueError(f"`rows` must be an integer tensor, got {rows.dtype}.")
+    if tuple(rows.shape) != (B,):
+        raise ValueError(f"`rows` must have shape (B,) = ({B},), got {tuple(rows.shape)}.")
+    if B:
+        if int(rows.min().item()) < 1:
+            raise ValueError("`rows` must be at least 1 for every problem.")
+        if int(rows.max().item()) > 2 ** 31 - 1:
+            raise ValueError("`rows` exceeds the number of residuals.")
+    return rows.to(device=dev, dtype=torch.int32).contiguous()
 
 
 _COPY_STREAM = {}

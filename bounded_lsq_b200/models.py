@@ -23,8 +23,14 @@ def _t_on(model, dev, cache):
     return t
 
 
-def callbacks(model_name, jac_kind="exact", lib=None):
-    """(fun, jac) for ``least_squares_batched(..., args=(PerProblem(y),))``."""
+def callbacks(model_name, jac_kind="exact", lib=None, rows=False):
+    """(fun, jac) for ``least_squares_batched(..., args=(PerProblem(y),))``.
+
+    ``rows=True`` (ExpDecay2, ragged batches): the callbacks take the
+    per-problem residual counts as a second argument,
+    ``args=(PerProblem(y), PerProblem(rows))`` with ``options={'rows': rows}``,
+    and write f and J only for the rows r < rows[b]; the padding of the (A, m)
+    and (A, m, 4) outputs is left unwritten (the solver never reads it)."""
     lib = lib or L.get_lib()
     if not lib.has("blsq_model_expdecay2"):
         raise L.BlsqError("library built without blsq_models.cu")
@@ -32,35 +38,45 @@ def callbacks(model_name, jac_kind="exact", lib=None):
     tcache = {}
     last = {}
     inlined = jac_kind == "inlined"
+    if rows and (model_name != "ExpDecay2" or inlined):
+        raise ValueError("rows-aware callbacks exist for ExpDecay2 with "
+                         "jac_kind 'exact' or a finite-difference scheme")
 
     if model_name == "ExpDecay2":
-        def run(X, idx, y, want_j):
+        def run(X, idx, y, want_j, nrows=None):
             A = X.shape[0]
             t = _t_on(model, X.device, tcache)
             F = torch.empty((A, model.m), dtype=torch.float64, device=X.device)
             J = torch.empty((A, model.m, 4), dtype=torch.float64,
                             device=X.device) if want_j else None
-            lib.call("blsq_model_expdecay2", A,
-                     None if idx is None else idx.data_ptr(), model.m,
-                     t.data_ptr(), X.data_ptr(), y.data_ptr(), F.data_ptr(),
-                     None if J is None else J.data_ptr(), lib.stream(X))
+            ip = None if idx is None else idx.data_ptr()
+            jp = None if J is None else J.data_ptr()
+            if nrows is None:
+                lib.call("blsq_model_expdecay2", A, ip, model.m, t.data_ptr(),
+                         X.data_ptr(), y.data_ptr(), F.data_ptr(), jp, lib.stream(X))
+            else:
+                if nrows.dtype != torch.int32:
+                    raise ValueError("rows-aware callbacks take int32 `rows`")
+                lib.call("blsq_model_expdecay2_rows", A, ip, model.m, t.data_ptr(),
+                         X.data_ptr(), y.data_ptr(), nrows.data_ptr(), F.data_ptr(), jp,
+                         lib.stream(X))
             return F, J
 
-        def fun(X, idx, y):
+        def fun(X, idx, y, nrows=None):
             # F and J come out of one kernel; J is handed to the `jac` call
             # that follows for the same X and dropped otherwise (the cache
             # never outlives the next callback: 2 GB at the C2 batch size)
-            F, J = run(X, idx, y, jac_kind == "exact" and not inlined)
+            F, J = run(X, idx, y, jac_kind == "exact" and not inlined, nrows)
             last.clear()
             if J is not None:
                 last[(X.data_ptr(), X.shape[0])] = J
             return F
 
-        def jac(X, idx, y):
+        def jac(X, idx, y, nrows=None):
             J = last.pop((X.data_ptr(), X.shape[0]), None)
             last.clear()
             if J is None:
-                _, J = run(X, idx, y, True)
+                _, J = run(X, idx, y, True, nrows)
             return J
 
     elif model_name == "GaussPeak":

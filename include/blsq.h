@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define BLSQ_VERSION 100
+#define BLSQ_VERSION 101
 
 #define BLSQ_E_BADARG (-1)      /* null pointer / negative size */
 #define BLSQ_E_UNSUPPORTED (-2) /* n outside 1..BLSQ_MAX_BATCHED_N, ... */
@@ -168,6 +168,30 @@ int blsq_round_batched(int method, int64_t A, const int32_t* idx, int m, int n,
                        double ftol, double xtol, double gtol, int max_nfev,
                        int first, double* state, int32_t* istate, double* Xnew,
                        double* Xjac, int32_t* work, int32_t* count, void* stream);
+
+/* Ragged batches (version 101): the two calls above with a per-problem number
+ * of residuals.  rows (nullable, int32) is indexed by problem id like istate
+ * (idx[slot], or the slot when idx is null); problem pid has residuals
+ * 0 .. rows[pid]-1.  m stays the row stride of F, J and Fp_host[*]; rows past
+ * rows[pid] are never read and may hold anything (NaN included).  Each problem
+ * is solved as the reference solves the problem made of its first rows[pid]
+ * residuals: the cost, full_rank = m >= n and the smin > eps*m*smax test
+ * (trust_region.py:108-112), the Gauss-Newton certificate and dogbox's
+ * rcond = eps*max(m, n_free) use rows[pid].  The kernels clamp rows[pid] to
+ * [0, m] for memory safety; callers reject counts outside 1 .. m.  With
+ * rows = null both are the calls above, bit for bit. */
+int blsq_linearise_batched_rows(int64_t A, const int32_t* idx, int m, int n,
+                                const double* F, const double* J,
+                                const double* const* Fp_host, const double* dx,
+                                int jac_mode, const int32_t* istate, double* lin,
+                                const int32_t* rows, void* stream);
+int blsq_round_batched_rows(int method, int64_t A, const int32_t* idx, int m, int n,
+                            const double* lin, const double* x0, const double* lb,
+                            const double* ub, int bstride, const double* scaling,
+                            double ftol, double xtol, double gtol, int max_nfev,
+                            int first, double* state, int32_t* istate, double* Xnew,
+                            double* Xjac, int32_t* work, int32_t* count,
+                            const int32_t* rows, void* stream);
 
 /* dogbox.py:152-154,254: on_bound as the reference's int array (B x n) */
 int blsq_dogbox_on_bound(int64_t B, int n, const int32_t* istate,

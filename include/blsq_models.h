@@ -22,6 +22,13 @@ extern "C" {
 int blsq_model_expdecay2(int64_t A, const int64_t* idx, int m, const double* t,
                          const double* X, const double* y, double* F, double* J,
                          void* stream);
+/* Ragged batches: rows (nullable, int32, indexed by problem id like y) gives
+ * problem pid rows[pid] residuals; only rows r < rows[pid] of F and J are
+ * written (the rest of each (m) / (m, 4) block is left as it was) and only
+ * those rows of y are used.  rows = null: blsq_model_expdecay2. */
+int blsq_model_expdecay2_rows(int64_t A, const int64_t* idx, int m, const double* t,
+                              const double* X, const double* y, const int32_t* rows,
+                              double* F, double* J, void* stream);
 /* The same model compiled INTO the linearisation kernel: the lin records of
  * blsq_linearise_batched (include/blsq.h) for the A trial points X, without
  * F and J ever being written to memory.  idx: int32 problem ids of the slots
