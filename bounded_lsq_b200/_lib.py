@@ -78,6 +78,14 @@ def _ptr(t):
     return t.data_ptr()
 
 
+def aligned(t, nbytes):
+    """``t``, or a copy in a fresh allocation when its address is not a
+    multiple of ``nbytes``: the kernels move rows with 128- and 256-bit loads,
+    and a contiguous view (e.g. J carved out of one buffer with F) can start
+    anywhere."""
+    return t if t.data_ptr() % nbytes == 0 else t.clone()
+
+
 class Lib:
     """Thin checked wrapper: tensors in, raw pointers out."""
 

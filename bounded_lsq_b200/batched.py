@@ -338,7 +338,7 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
                     raise RuntimeError(
                         "Inconsistent dimensions between the returns of `fun` "
                         "and `jac` on the first iteration.")
-                J = J.contiguous()
+                J = L.aligned(J.contiguous(), 32 if n % 4 == 0 else (16 if n % 2 == 0 else 8))
                 tock("callbacks", t0, nrun)
                 t0 = tick()
                 lin_call(A, ip, m, n, F.data_ptr(), J.data_ptr(), None, None, 0,

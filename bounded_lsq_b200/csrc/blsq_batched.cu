@@ -568,6 +568,10 @@ int blsq_linearise_batched_rows(int64_t A, const int32_t* idx, int m, int n,
     if (A < 0 || m < 1 || !F || !istate || !lin) return BLSQ_E_BADARG;
     if (jac_mode < 0 || jac_mode > 2) return BLSQ_E_BADARG;
     if (jac_mode == 0 && !J) return BLSQ_E_BADARG;
+    // lin_kernel loads the rows of J with 256-bit (n % 4 == 0) or 128-bit
+    // (n = 2, 6) vector loads: a misaligned J would fault the device
+    if (jac_mode == 0 && (uintptr_t)J % (n % 4 == 0 ? 32 : (n % 2 == 0 ? 16 : 8)))
+        return BLSQ_E_BADARG;
     if (jac_mode != 0 && (!dx || !Fp_host)) return BLSQ_E_BADARG;
     if (jac_mode != 0 && n >= 1 && n <= BLSQ_MAX_BATCHED_N)
         for (int j = 0; j < jac_mode * n; j++)

@@ -322,6 +322,7 @@ int blsq_model_expdecay2_linearise(int64_t A, const int32_t* idx, int m, const d
                                    double* lin, void* stream) {
     using namespace blsq_lin;
     if (A < 0 || m < 1 || !t || !X || !y || !istate || !lin) return BLSQ_E_BADARG;
+    if ((uintptr_t)X % 32) return BLSQ_E_BADARG;                // double4 loads of X
     if (m > 8 * LinCfg<4>::RPL) return BLSQ_E_UNSUPPORTED;      // all rows in one lane group
     if (A == 0) return 0;
     ExpDecay2Rows mdl{t, X, y, m};
@@ -339,6 +340,8 @@ int blsq_model_expdecay2_rows(int64_t A, const int64_t* idx, int m, const double
                               const double* X, const double* y, const int32_t* rows,
                               double* F, double* J, void* stream) {
     if (A < 0 || m < 1 || !t || !X || !y || !F) return BLSQ_E_BADARG;
+    // double4 loads of X and 256-bit stores of the rows of J in every variant
+    if ((uintptr_t)X % 32 || (uintptr_t)J % 32) return BLSQ_E_BADARG;
     if (A == 0) return 0;
     dim3 block, grid;
     const bool quads = BLSQ_EXPDECAY2_QUADS && m % 4 == 0 && ((uintptr_t)t % 32 == 0) &&
@@ -385,6 +388,7 @@ int blsq_model_gausspeak(int64_t A, const int64_t* idx, int m, const double* t,
 int blsq_model_linexp_fun(int64_t m, int n, const double* J, const double* t,
                           const double* y, const double* x, double* F, void* stream) {
     if (m < 0 || n < 6 || n > 256 || (n & 1) || !J || !t || !y || !x || !F) return BLSQ_E_BADARG;
+    if ((uintptr_t)J % 16) return BLSQ_E_BADARG;               // 128-bit loads of J
     if (m == 0) return 0;
     int64_t blocks = (m + 255) / 256;
     if (blocks > 148 * 8) blocks = 148 * 8;
@@ -396,6 +400,7 @@ int blsq_model_linexp_fun(int64_t m, int n, const double* J, const double* t,
 int blsq_model_linexp_jac(int64_t m, int n, double* J, const double* t, const double* x,
                           void* stream) {
     if (m < 0 || n < 6 || n > 256 || (n & 1) || !J || !t || !x) return BLSQ_E_BADARG;
+    if ((uintptr_t)J % 16) return BLSQ_E_BADARG;               // 128-bit stores into J
     if (m == 0) return 0;
     int64_t blocks = (m + 255) / 256;
     if (blocks > 148 * 16) blocks = 148 * 16;

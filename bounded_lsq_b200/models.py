@@ -51,6 +51,7 @@ def callbacks(model_name, jac_kind="exact", lib=None, rows=False):
                             device=X.device) if want_j else None
             ip = None if idx is None else idx.data_ptr()
             jp = None if J is None else J.data_ptr()
+            X = L.aligned(X.contiguous(), 32)       # the kernels load X with double4
             if nrows is None:
                 lib.call("blsq_model_expdecay2", A, ip, model.m, t.data_ptr(),
                          X.data_ptr(), y.data_ptr(), F.data_ptr(), jp, lib.stream(X))

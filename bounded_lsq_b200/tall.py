@@ -135,7 +135,8 @@ def solve_tall(lib, method, fun, jac, x0, lb, ub, ftol, xtol, gtol, max_nfev,
             f = f.reshape(1)
         if f.dim() > 1:
             raise RuntimeError("`fun` must return at most 1-d array_like.")
-        return f.to(f64).contiguous()
+        # blsq_tall_gram moves rows with 16-byte bulk copies
+        return L.aligned(f.to(f64).contiguous(), 16)
 
     def call_jac(x, f):
         if callable(jac):
@@ -149,7 +150,7 @@ def solve_tall(lib, method, fun, jac, x0, lb, ub, ftol, xtol, gtol, max_nfev,
             J = J.to(f64)
         else:
             J = _fd_jacobian_tall(lib, call_fun, x, f, lb, ub, diff_step, st, jac)
-        return J if J.is_contiguous() else J.contiguous()
+        return L.aligned(J.contiguous(), 16)
 
     state = torch.zeros(lay["state_size"], dtype=f64, device=dev)
     istate = torch.zeros(lay["istate_size"], dtype=torch.int32, device=dev)

@@ -135,7 +135,13 @@ int blsq_init_batched(int method, int64_t B, int n, const double* x0,
  *   jac_mode 2: 3-point: Fp_host holds 2n device pointers in the batch order
  *               of blsq_fd3_points, dx is its (A, 2n) dxo array;
  *               J[:, i] = (f2 - f1) / dx_i or (-3 f + 4 f1 - f2) / dx_i.
- * Slots whose problem is no longer running are skipped. */
+ * Slots whose problem is no longer running are skipped.
+ * Alignment (jac_mode 0): the rows of J are read with vector loads, so J must
+ * be 32-byte aligned for n = 4, 8 and 16-byte aligned for n = 2, 6; otherwise
+ * BLSQ_E_BADARG before any launch.
+ * Valid range: sums of squares are formed in double, so every squared column
+ * norm of [J | f] must be a normal double (entries between about 2^-500 and
+ * 2^500 at m <= 1100); outside it the record is inaccurate or not finite. */
 int blsq_linearise_batched(int64_t A, const int32_t* idx, int m, int n,
                            const double* F, const double* J,
                            const double* const* Fp_host, const double* dx,

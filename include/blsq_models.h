@@ -18,7 +18,9 @@
 extern "C" {
 #endif
 
-/* y = a e^{-b t} + c e^{-d t}: F (A, m) = model - y[idx]; J (A, m, 4) or null */
+/* y = a e^{-b t} + c e^{-d t}: F (A, m) = model - y[idx]; J (A, m, 4) or null.
+ * X and J must be 32-byte aligned (double4 loads, 256-bit stores), else
+ * BLSQ_E_BADARG; so must X of blsq_model_expdecay2_linearise. */
 int blsq_model_expdecay2(int64_t A, const int64_t* idx, int m, const double* t,
                          const double* X, const double* y, double* F, double* J,
                          void* stream);
@@ -43,7 +45,8 @@ int blsq_model_gausspeak(int64_t A, const int64_t* idx, int m, const double* t,
 /* tall workload (C4/C5): J (m, n) keeps the constant design matrix in its
  * first n-4 columns; x is a DEVICE pointer to n doubles.
  *   fun: F = J[:, :n-4] x[:n-4] + x_k e^{-x_{k+1} t} + x_{k+2} e^{-x_{k+3} t} - y
- *   jac: rewrites columns n-4..n-1 of J for the point x */
+ *   jac: rewrites columns n-4..n-1 of J for the point x
+ * J must be 16-byte aligned (128-bit loads and stores), else BLSQ_E_BADARG. */
 int blsq_model_linexp_fun(int64_t m, int n, const double* J, const double* t,
                           const double* y, const double* x, double* F,
                           void* stream);
