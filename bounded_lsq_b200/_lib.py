@@ -62,7 +62,7 @@ SIGNATURES = {
 METHOD_TRF = 0
 METHOD_DOGBOX = 1
 ISTATE_SIZE = 8
-MAX_BATCHED_N = 8
+MAX_BATCHED_N = 16                 # BLSQ_MAX_BATCHED_N
 STATUS_RUNNING = -1
 STATUS_ERR_TR_ZERO = -101
 STATUS_ERR_TR_OUTSIDE = -102

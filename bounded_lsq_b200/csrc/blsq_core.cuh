@@ -1144,12 +1144,15 @@ struct DogState {
     static constexpr int SIZE = OBJ + 5;
 };
 
+// The fields are shifted as unsigned: coordinate 15 owns bits 30-31, and
+// 2 << 30 on a signed int (or a right shift of a negative word) is not well
+// defined.
 BLSQ_HD int get2(int word, int i) {      // decode 2-bit field -> -1/0/+1
-    int v = (word >> (2 * i)) & 3;
-    return v == 1 ? -1 : (v == 2 ? 1 : 0);
+    unsigned v = ((unsigned)word >> (2 * i)) & 3u;
+    return v == 1u ? -1 : (v == 2u ? 1 : 0);
 }
 BLSQ_HD int put2(int i, int val) {       // val in -1/0/+1
-    return (val < 0 ? 1 : (val > 0 ? 2 : 0)) << (2 * i);
+    return (int)((unsigned)(val < 0 ? 1 : (val > 0 ? 2 : 0)) << (2 * i));
 }
 
 // dogleg_step / constrained_cauchy_step over the free coordinates

@@ -41,9 +41,27 @@ struct NoModel {
 #ifndef BLSQ_LIN_MINB_MID
 #define BLSQ_LIN_MINB_MID 3
 #endif
-template <int N> struct LinCfg {
+template <int N, bool WIDE = (N > 8)> struct LinCfg {
     static constexpr int RPL = (N <= 4) ? BLSQ_RPL_SMALL : (N <= 6 ? BLSQ_RPL_MID : 4);
     static constexpr int MINB = (N <= 4 || RPL <= 4) ? BLSQ_LIN_MINB : BLSQ_LIN_MINB_MID;
+};
+// N = 9..16 (blsq_batched_wide.cu; lane groups of 16 / 32 only): 4 rows per
+// lane up to N = 12, then 2, at 2 CTAs / SM (255 registers).  The largest
+// budgets without spills in any of the 18 instances of an N: 4 rows at 3 CTAs
+// spill 1.3-1.5 KB at N = 12 in MULTI, 4 rows spill at N = 16 even at 2 CTAs
+// (profiles/r4_wide_ptxas.md).
+#ifndef BLSQ_RPL_WIDE
+#define BLSQ_RPL_WIDE 4
+#endif
+#ifndef BLSQ_RPL_WIDE_TO
+#define BLSQ_RPL_WIDE_TO 12
+#endif
+#ifndef BLSQ_LIN_MINB_WIDE
+#define BLSQ_LIN_MINB_WIDE 2
+#endif
+template <int N> struct LinCfg<N, true> {
+    static constexpr int RPL = N <= BLSQ_RPL_WIDE_TO ? BLSQ_RPL_WIDE : 2;
+    static constexpr int MINB = BLSQ_LIN_MINB_WIDE;
 };
 
 template <int G>
@@ -270,6 +288,14 @@ lin_kernel(int64_t A, const int32_t* __restrict__ idx, int m,
             }
             double rkk, inv_rkk, inv_dk;
             norm_terms(dts[k], rkk, inv_rkk, inv_dk);
+            // N > 8: with m << N, a column that depends on the ones before it
+            // keeps only rounding residue, which shrinks by ~u per projection;
+            // after ten of them its squared norm is subnormal and inv_dk = 1/d
+            // overflows.  Such a column is treated as dependent, as d <= 0 is
+            if (N > 8 && !(dts[k] >= 2.2250738585072014e-308)) {
+                inv_rkk = 0.0;
+                inv_dk = 0.0;
+            }
             if (MULTI) {
                 if (lane == k) {
 #pragma unroll

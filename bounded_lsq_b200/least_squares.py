@@ -132,7 +132,8 @@ def least_squares_batched(fun, x0, jac='2-point', bounds=(-float('inf'), float('
                           _lib=None):
     """Solve B independent bounded problems (same n, m, method, tolerances).
 
-    x0 : (B, n).  bounds : scalars, (n,) or (B, n) tensors.
+    x0 : (B, n) with 1 <= n <= 16 (ValueError beyond).  bounds : scalars, (n,)
+    or (B, n) tensors.
     fun(X, *args, **kwargs) -> (A, m) and jac(X, *args, **kwargs) -> (A, m, n)
     are called on the A <= B problems still running (rows in problem order);
     wrap per-problem tensors in ``PerProblem`` so they are gathered alike.
@@ -408,9 +409,13 @@ def _stage_host_inputs(x0, args, kwargs, options):
     return stage_host_inputs(x0, args, kwargs, device=dev, h2d_chunks=nch)
 
 
-# A single problem with n <= 8 goes to the batched kernels (B = 1) unless it is
-# tall: from this many rows on, the row-sharded Gram kernels of tall mode
-# (n >= 2) are the faster path -- one warp folding m rows chunk by chunk is not.
+# A single problem with n <= SINGLE_BATCHED_MAX_N goes to the batched kernels
+# (B = 1) unless it is tall: from TALL_FROM_ROWS rows on, the row-sharded Gram
+# kernels of tall mode (n >= 2) are the faster path -- one warp folding m rows
+# chunk by chunk is not.  Batched mode takes n up to L.MAX_BATCHED_N = 16, but
+# a single problem with 9 <= n <= 16 stays on the tall kernels unless
+# options={'mode': 'batched'} asks for them.
+SINGLE_BATCHED_MAX_N = 8
 TALL_FROM_ROWS = 32768
 
 
@@ -467,13 +472,13 @@ def least_squares(fun, x0, jac='2-point', bounds=(-float('inf'), float('inf')),
     the field's documented meaning (least_squares.py:248-252: the inverse of
     J^T J at the solution) from the triangular factor the solve already holds.
 
-    Kernels: n <= 8 runs on the batched kernels (B = 1) and n > 8 on the tall
-    ones; a problem with 2 <= n <= 8 and TALL_FROM_ROWS or more residuals is
-    moved to the tall kernels after its first residual evaluation (that one
-    call is repeated; the solve is then local to this process).
-    ``options={'mode': 'batched' | 'tall'}`` pins the choice; with
-    ``mode='tall'`` and an initialised process group the callbacks return this
-    rank's rows, as for n > 8.
+    Kernels: n <= 8 (SINGLE_BATCHED_MAX_N) runs on the batched kernels (B = 1)
+    and n > 8 on the tall ones; a problem with 2 <= n <= 8 and TALL_FROM_ROWS
+    or more residuals is moved to the tall kernels after its first residual
+    evaluation (that one call is repeated; the solve is then local to this
+    process).  ``options={'mode': 'batched' | 'tall'}`` pins the choice
+    (batched: n <= 16); with ``mode='tall'`` and an initialised process group
+    the callbacks return this rank's rows, as for n > 8.
     """
     lib = _lib if _lib is not None else L.get_lib()
     _validate_common(method, bounds, jac)
@@ -508,7 +513,7 @@ def _least_squares(lib, fun, x0, jac, bounds, method, ftol, xtol, gtol, max_nfev
         raise ValueError("`x0` is infeasible.")
 
     # options['mode'] = 'batched' | 'tall' pins the kernels; by default n and
-    # (for 2 <= n <= 8) the number of residuals decide
+    # (for 2 <= n <= SINGLE_BATCHED_MAX_N) the number of residuals decide
     options = dict(options)
     mode = options.pop("mode", None)
     if mode not in (None, "batched", "tall"):
@@ -523,7 +528,7 @@ def _least_squares(lib, fun, x0, jac, bounds, method, ftol, xtol, gtol, max_nfev
         return solve_tall(lib, method, fun, jac, x0, lb, ub, ftol, xtol, gtol,
                           max_nfev, scaling, diff_step, args, kwargs, options)
 
-    if n > L.MAX_BATCHED_N or mode == "tall":
+    if mode == "tall" or (mode is None and n > SINGLE_BATCHED_MAX_N):
         return tall()
 
     probe = TALL_FROM_ROWS if (mode is None and n >= 2 and

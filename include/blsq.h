@@ -27,12 +27,14 @@
 extern "C" {
 #endif
 
-#define BLSQ_VERSION 101
+#define BLSQ_VERSION 102
 
 #define BLSQ_E_BADARG (-1)      /* null pointer / negative size */
 #define BLSQ_E_UNSUPPORTED (-2) /* n outside 1..BLSQ_MAX_BATCHED_N, ... */
 
-#define BLSQ_MAX_BATCHED_N 8
+/* batched mode takes 1 <= n <= 16 (version 102; 8 before): istate packs two
+ * bits per coordinate in one int32 (dogbox's on_bound and bound marks) */
+#define BLSQ_MAX_BATCHED_N 16
 
 #define BLSQ_METHOD_TRF 0
 #define BLSQ_METHOD_DOGBOX 1
@@ -137,8 +139,8 @@ int blsq_init_batched(int method, int64_t B, int n, const double* x0,
  *               J[:, i] = (f2 - f1) / dx_i or (-3 f + 4 f1 - f2) / dx_i.
  * Slots whose problem is no longer running are skipped.
  * Alignment (jac_mode 0): the rows of J are read with vector loads, so J must
- * be 32-byte aligned for n = 4, 8 and 16-byte aligned for n = 2, 6; otherwise
- * BLSQ_E_BADARG before any launch.
+ * be 32-byte aligned for n = 4, 8, 12, 16 and 16-byte aligned for n = 2, 6, 10,
+ * 14; otherwise BLSQ_E_BADARG before any launch.
  * Valid range: sums of squares are formed in double, so every squared column
  * norm of [J | f] must be a normal double (entries between about 2^-500 and
  * 2^500 at m <= 1100); outside it the record is inaccurate or not finite. */
