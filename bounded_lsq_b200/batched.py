@@ -20,7 +20,6 @@ from __future__ import annotations
 
 import ctypes as C
 import os
-import sys
 import warnings
 
 import torch
@@ -63,15 +62,18 @@ class BatchedCallbacks:
         self.B = B
         self._gathered = (None, None)     # (idx, gathered args) of the last call
 
+    def _raw_args(self, sl):
+        """args / kwargs with every per-problem tensor sliced to ``sl`` but not
+        gathered: the indexed callbacks take the active ids themselves."""
+        def raw(v):
+            return v.tensor[sl] if isinstance(v, PerProblem) else v
+        return (tuple(raw(v) for v in self.args),
+                {n: raw(v) for n, v in self.kwargs.items()})
+
     def _call(self, fn, X, idx):
         if getattr(fn, "blsq_indexed", False):
             # indexed protocol: raw per-problem tensors + the active ids
-            sl = idx if isinstance(idx, slice) else slice(None)
-
-            def raw(v):
-                return v.tensor[sl] if isinstance(v, PerProblem) else v
-            a = tuple(raw(v) for v in self.args)
-            k = {n: raw(v) for n, v in self.kwargs.items()}
+            a, k = self._raw_args(idx if isinstance(idx, slice) else slice(None))
             return fn(X, None if isinstance(idx, slice) else idx, *a, **k)
         # the active set only changes when the driver compacts it: gather the
         # per-problem data once per compaction, not once per callback
@@ -88,11 +90,7 @@ class BatchedCallbacks:
         if fn is None:
             return None
         sl = slice(off, off + A) if (idx32 is None and (off or A != self.B)) else slice(None)
-
-        def raw(v):
-            return v.tensor[sl] if isinstance(v, PerProblem) else v
-        a = tuple(raw(v) for v in self.args)
-        k = {n: raw(v) for n, v in self.kwargs.items()}
+        a, k = self._raw_args(sl)
         return fn(X, idx32, p_istate, p_lin, stream, *a, **k)
 
     def f(self, X, idx):
@@ -109,21 +107,6 @@ def _side_stream(dev):
     s = _SIDE.get(dev)
     if s is None:
         s = _SIDE[dev] = torch.cuda.Stream(dev)
-    return s
-
-
-_CSTREAM = {}
-
-
-def _count_stream(dev):
-    """Side stream, pinned landing buffer and events of the look-ahead status
-    polls (4-byte copies), one set per device."""
-    s = _CSTREAM.get(dev)
-    if s is None:
-        s = _CSTREAM[dev] = (torch.cuda.Stream(dev),
-                             torch.zeros(2, dtype=torch.int32).pin_memory(),
-                             [torch.cuda.Event(), torch.cuda.Event()],
-                             [torch.cuda.Event(), torch.cuda.Event()])
     return s
 
 
@@ -172,7 +155,7 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
                   max_nfev, scaling, diff_step=None, check_every=2,
                   compact_below=0.75, tail_below=8192, trace=None,
                   timers=None, graph_tail_rounds=None, prologue=None,
-                  prologue_rounds=6, x_covariance=False, lookahead=None, rows=None):
+                  prologue_rounds=6, x_covariance=False, rows=None):
     """Run ``method`` ('trf' | 'dogbox') on B problems.
 
     fun(X, idx) -> (A, m); jac is a callable jac(X, idx) -> (A, m, n) or the
@@ -223,12 +206,10 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
     # count[2] = problems still running after the last round (written by the
     # round kernel itself, blsq_round_batched `count`)
     count = torch.zeros(4, dtype=torch.int32, device=dev)
-    # BLSQ_ROUND_COUNT=0: count with the separate blsq_count_running launch
-    fused_count = os.environ.get("BLSQ_ROUND_COUNT", "1") != "0"
     # TRF: worklist of the problems that leave the Gauss-Newton shortcut
-    # (blsq_round_batched `work`); BLSQ_TRF_TWO_KERNELS=0 -> single kernel
+    # (blsq_round_batched `work`)
     rwork = None
-    if method == "trf" and os.environ.get("BLSQ_TRF_TWO_KERNELS", "1") != "0":
+    if method == "trf":
         rwork = torch.empty(B + 1, dtype=torch.int32, device=dev)
     rwork_ptr = None if rwork is None else rwork.data_ptr()
     # latency-sized rounds are faster as ONE kernel (measured: the second
@@ -369,19 +350,12 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
                    float(ftol), float(xtol), float(gtol), max_nfev, first,
                    p_st, p_ist, p_xn, p_xj,
                    rwork_ptr if A >= TWO_KERNELS_ABOVE else None,
-                   count.data_ptr() if (count_here and fused_count) else None, p_rows, stream)
+                   count.data_ptr() if count_here else None, p_rows, stream)
         tock("round", t0, nrun)
         if timers is not None:
             timers["shape"] = (n, m, LS, S)
         launches += (2 if (rwork is None or A < TWO_KERNELS_ABOVE) else 3) - \
             (1 if mm is not None else 0)
-
-    def count_separately(A, idx32):
-        nonlocal launches
-        lib.call("blsq_count_running", A,
-                 None if idx32 is None else idx32.data_ptr(),
-                 istate.data_ptr(), count[2:].data_ptr(), lib.stream(X0))
-        launches += 1
 
     def graph_tail(A, idx, idx32, nrun):
         """The latency-sized tail of the batch (A <= tail_below slots, often a
@@ -400,14 +374,10 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
         # allocator on entry (every later allocation of the batch would go
         # back to cudaMalloc); capture_begin / capture_end on a side stream
         # do neither.
-        dbg = os.environ.get("BLSQ_GRAPH_DEBUG")
         # drain the (latency-sized) queue first: measured on the B200, a
         # capture that starts while the eager round is still in flight costs
         # ~16 ms more per solve than the microseconds this wait takes
         torch.cuda.current_stream(dev).synchronize()
-        if dbg:
-            import time
-            tt = [time.perf_counter()]
         g = torch.cuda.CUDAGraph()
         cur = torch.cuda.current_stream(dev)
         side = _side_stream(dev)
@@ -418,21 +388,13 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
                 # keep making CUDA calls during the capture
                 g.capture_begin(pool=_graph_pool(dev),
                                 capture_error_mode="thread_local")
-                if dbg:
-                    tt.append(time.perf_counter())
                 try:
                     for _ in range(GRAPH_ROUNDS):
                         one_round(A, idx, idx32, 0, nrun)
-                    if not fused_count:
-                        count_separately(A, idx32)
                 finally:
-                    if dbg:
-                        tt.append(time.perf_counter())
                     g.capture_end()
             cur.wait_stream(side)
             _LAST_GRAPH[dev] = g
-            if dbg:
-                tt.append(time.perf_counter())
         except Exception as e:                 # noqa: BLE001
             torch.cuda.synchronize(dev)
             # a capture that died half way leaves the allocator routing this
@@ -456,12 +418,6 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
             launches += per_replay
             r += GRAPH_ROUNDS
             if int(count[2].item()) == 0 or rounds + r > max_nfev + 1:
-                if dbg:
-                    tt.append(time.perf_counter())
-                    print("# graph tail A=%d: begin %.2f capture %.2f end %.2f "
-                          "replays(%d rounds) %.2f ms" % (
-                              A, *[(b - a) * 1e3 for a, b in zip(tt, tt[1:])][:3],
-                              r, (tt[-1] - tt[-2]) * 1e3), file=sys.stderr)
                 return r, True
 
     if graph_tail_rounds is None:                  # BLSQ_GRAPH_TAIL=0 turns it off
@@ -488,10 +444,11 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
                           count_here=False)
         first = 0
         rounds = K
-    def compact(A, idx32, nrun_hint):
+
+    def compact(A, idx32, nrun):
         """Ordered compaction on the device (3 small launches) into the other
-        half of a ping-pong pair; returns the exact number of survivors (one
-        blocking read: compactions are ~10 per solve)."""
+        half of a ping-pong pair; the nrun problems still running (the round
+        kernel's count) fill its first slots."""
         nonlocal pong, flip, cwork, launches, Xnew, Xjac
         if pong is None:
             pong = [dict(X=torch.empty_like(Xnew),
@@ -515,70 +472,9 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
                  cwork.data_ptr(), lib.stream(X0))
         launches += 3
         Xnew, Xjac = o["X"], o["J"]
-        if nrun_hint is None:
-            ntot = int(cwork[int(lib._dll.blsq_compact_work_size(A)) - 1].item())
-        else:
-            ntot = nrun_hint
-        return ntot, o["i64"][:ntot], o["i32"][:ntot]
+        return nrun, o["i64"][:nrun], o["i32"][:nrun]
 
-    # Look-ahead polling (CUDA): round r + 1 is queued BEFORE the host waits for
-    # the running count of round r (copied to pinned memory on a side stream),
-    # so the GPU never idles on a host look; the count that triggers a
-    # compaction is one round old, the compaction itself reports the exact
-    # number of survivors.  The synchronous form is kept for the trace hook,
-    # for BLSQ_ROUND_COUNT=0 and for the host emulation of the tests.
-    # Measured on one B200 the look-ahead form is 0.7 ms per C2 solve SLOWER than
-    # a blocking look every second round (19.5 ms): the GPU is never idle there
-    # anyway and every compaction comes one round later.  It is meant for many
-    # driver processes on one host (8 GPUs), hence opt-in (option `lookahead`
-    # or BLSQ_LOOKAHEAD=1).
-    if lookahead is None:
-        lookahead = os.environ.get("BLSQ_LOOKAHEAD", "0") == "1"
-    lookahead = bool(lookahead) and X0.is_cuda and fused_count and trace is None
-    if lookahead:
-        cnt2 = [count, torch.zeros(4, dtype=torch.int32, device=dev)]
-        cside, hcnt, ev_done, ev_copy = _count_stream(dev)
-        look = None
-        main_count = count
-        while A > 0:
-            s_ = rounds & 1
-            count = cnt2[s_]                       # the slot this round reports into
-            one_round(A, idx, idx32, first, nrun)
-            main = torch.cuda.current_stream(dev)
-            ev_done[s_].record(main)
-            with torch.cuda.stream(cside):
-                cside.wait_event(ev_done[s_])
-                hcnt[s_:s_ + 1].copy_(count[2:3], non_blocking=True)
-                ev_copy[s_].record(cside)
-            first = 0
-            rounds += 1
-            prev, look = look, s_
-            if prev is None and rounds < max_nfev:
-                continue
-            if prev is None:                       # budget exhausted on the first look
-                prev, look = s_, None
-            ev_copy[prev].synchronize()            # waits for the round BEFORE the one in flight
-            nrun = int(hcnt[prev])
-            if nrun == 0:
-                break
-            if nrun <= compact_below * A:
-                A, idx, idx32 = compact(A, idx32, None)
-                nrun = A
-                look = None                        # counts in flight refer to the old slots
-                if A == 0:
-                    break
-            if use_graph and A <= tail_below:
-                count = main_count
-                r, done = graph_tail(A, idx, idx32, nrun)
-                rounds += r
-                if done:
-                    break
-                use_graph = False                  # not capturable: eager
-                look = None
-            if rounds > max_nfev + 3:              # cannot happen
-                raise RuntimeError("batched driver failed to terminate")
-        count = main_count
-    while not lookahead and A > 0:
+    while A > 0:
         one_round(A, idx, idx32, first, nrun)
         first = 0
         rounds += 1
@@ -588,8 +484,6 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
         # are bandwidth-sized, every 4th once they are launch-latency sized
         every = check_every if A > tail_below else max(check_every, 4)
         if rounds % every == 0 or rounds >= max_nfev:
-            if not fused_count:
-                count_separately(A, idx32)
             nrun = int(count[2].item())               # the one host sync
             if nrun == 0:
                 break

@@ -546,7 +546,7 @@ def _least_squares(lib, fun, x0, jac, bounds, method, ftol, xtol, gtol, max_nfev
         # evaluation at x0 was spent to learn m)
         options.pop("graph_tail_rounds", None)
         for k in ("check_every", "compact_below", "tail_below", "prologue",
-                  "prologue_rounds", "lookahead"):
+                  "prologue_rounds"):
             options.pop(k, None)
         # the decision was taken from this process's rows alone, so the solve
         # is local too; rows sharded over ranks need mode='tall' (or n > 8)

@@ -17,9 +17,7 @@ lb, ub = torch.as_tensor(model.lb, device=dev), torch.as_tensor(model.ub, device
 fun, jac = models.callbacks("ExpDecay2", "exact")
 
 
-def run(label, env=None, **opts):
-    for k, v in (env or {}).items():
-        os.environ[k] = v
+def run(label, **opts):
     ts = []
     for i in range(8):
         torch.cuda.synchronize()
@@ -31,8 +29,6 @@ def run(label, env=None, **opts):
         e1.record()
         torch.cuda.synchronize()
         ts.append((round((time.perf_counter() - t0) * 1e3, 2), round(e0.elapsed_time(e1), 2)))
-    for k in (env or {}):
-        os.environ.pop(k)
     print(json.dumps(dict(variant=label, wall_event_ms=ts, rounds=r.rounds,
                           launches=r.kernel_launches)), flush=True)
 
@@ -52,9 +48,7 @@ if os.environ.get("SWEEP"):
     sys.exit(0)
 
 run("default")
-run("separate count kernel", env={"BLSQ_ROUND_COUNT": "0"})
 run("no graph tail", graph_tail_rounds=0)
-run("one kernel per TRF round", env={"BLSQ_TRF_TWO_KERNELS": "0"})
 run("prologue 7 rounds (no count, no host look)", prologue=[(0, B, None)], prologue_rounds=7)
 run("check every 2 rounds", check_every=2)
 run("no compaction", compact_below=0.0)
