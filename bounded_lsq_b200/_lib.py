@@ -42,6 +42,8 @@ SIGNATURES = {
     "blsq_linearise_batched_rows": [_l, _p, _i, _i, _p, _p, _p, _p, _i, _p, _p, _p, _p],
     "blsq_round_batched_rows": [_i, _l, _p, _i, _i, _p, _p, _p, _p, _i, _p,
                                 _d, _d, _d, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p],
+    "blsq_linearise_batched_ld": [_l, _p, _i, _i, _i, _p, _p, _p, _p, _i, _p, _p, _p, _p],
+    "blsq_pad_points": [_i, _p, _l, _i, _i, _p, _p],
     "blsq_dogbox_on_bound": [_l, _i, _p, _p, _p],
     "blsq_count_running": [_l, _p, _p, _p, _p],
     "blsq_model_expdecay2": [_l, _p, _i, _p, _p, _p, _p, _p, _p],
@@ -58,6 +60,13 @@ SIGNATURES = {
     "blsq_tall_round": [_i, _i, _i, _l, _i, _p, _p, _p, _p, _p, _p, _d, _d, _d,
                         _i, _i, _i, _p, _p, _p, _p],
 }
+
+
+class PadSegment(C.Structure):
+    """blsq_pad_segment (include/blsq.h)."""
+    _fields_ = [("off", C.c_int64), ("A", C.c_int64), ("n", C.c_int), ("idx", _p),
+                ("x0", _p), ("X", _p), ("Xp", _p)]
+
 
 METHOD_TRF = 0
 METHOD_DOGBOX = 1

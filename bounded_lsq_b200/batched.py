@@ -151,11 +151,18 @@ def _as_f64(t, like, what):
     return t
 
 
+class _Segment:
+    """The problems of one parameter count N: a dense lock-step solve of its
+    own (state and lin records, istate, active set, count buffer, compaction)
+    whose active slots are one contiguous range of every round's callback
+    batch."""
+
+
 def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
                   max_nfev, scaling, diff_step=None, check_every=2,
                   compact_below=0.75, tail_below=8192, trace=None,
                   timers=None, graph_tail_rounds=None, prologue=None,
-                  prologue_rounds=6, x_covariance=False, rows=None):
+                  prologue_rounds=6, x_covariance=False, rows=None, cols=None):
     """Run ``method`` ('trf' | 'dogbox') on B problems.
 
     fun(X, idx) -> (A, m); jac is a callable jac(X, idx) -> (A, m, n) or the
@@ -164,6 +171,17 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
     has residuals 0 .. rows[b]-1 of the (A, m) callback outputs (ragged batch,
     blsq_linearise_batched_rows / blsq_round_batched_rows).  Returns a dict
     of device tensors (see least_squares_batched).
+
+    cols: None, or an int32 (B,) tensor on X0's device with 1 <= cols[b] <= n
+    -- problem b has parameters 0 .. cols[b]-1, the others are held at
+    X0[b].  The problems are permuted once into segment-major order (a stable
+    sort on cols), and each distinct count N is a *segment*: a dense solve
+    of N-parameter problems run by the dense N kernels.  The segments share
+    one callback call per round: blsq_pad_points writes their active points
+    into one padded (A, n) batch (segment after segment, so the callbacks get
+    the original problem ids as idx), and each segment linearises its slots
+    of the outputs in place (blsq_linearise_batched_ld).  Without cols the
+    batch is one segment and the calls are those of a dense solve.
     """
     meth = {"trf": L.METHOD_TRF, "dogbox": L.METHOD_DOGBOX}[method]
     dev = X0.device
@@ -175,19 +193,12 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
     lib.check_tensor(lb, f64, "lb")
     lib.check_tensor(ub, f64, "ub")
     bstride = 0 if lb.dim() == 1 else n
-    lay = lib.state_layout(meth, n)
-    S = lay["size"]
-    LS = lib.lin_record_size(n)
-    if max_nfev is None:
-        max_nfev = 100 * n                           # trf.py:234-235
-    max_nfev = int(max_nfev)
     jac_scaling = isinstance(scaling, str)
     sc_ptr = None if jac_scaling else scaling.data_ptr()
     if not jac_scaling:
         lib.check_tensor(scaling, f64, "scaling")
     fd = isinstance(jac, str)
     fd3 = fd and jac == '3-point'
-    npts = 2 * n if fd3 else n                       # callback calls per FD Jacobian
     rel = float("nan") if diff_step is None else float(diff_step)
     rows_max = None
     if rows is not None:
@@ -195,35 +206,88 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
         if rows.shape != (B,):
             raise ValueError("`rows` must have shape (B,).")
         rows_max = int(rows.max().item()) if B else 0
+    padded = cols is not None
+    if padded:
+        lib.check_tensor(cols, torch.int32, "cols")
+        if cols.shape != (B,):
+            raise ValueError("`cols` must have shape (B,).")
 
-    state = torch.zeros((B, S), dtype=f64, device=dev)
-    istate = torch.zeros((B, L.ISTATE_SIZE), dtype=torch.int32, device=dev)
-    Xnew = torch.empty((B, n), dtype=f64, device=dev)
-    # dogbox evaluates J at the bound-snapped trial (dogbox.py:256-261)
-    Xjac = torch.empty((B, n), dtype=f64, device=dev) if method == "dogbox" \
-        else None
-    lin = torch.empty((B, LS), dtype=f64, device=dev)
-    # count[2] = problems still running after the last round (written by the
-    # round kernel itself, blsq_round_batched `count`)
-    count = torch.zeros(4, dtype=torch.int32, device=dev)
-    # TRF: worklist of the problems that leave the Gauss-Newton shortcut
-    # (blsq_round_batched `work`)
-    rwork = None
-    if method == "trf":
-        rwork = torch.empty(B + 1, dtype=torch.int32, device=dev)
-    rwork_ptr = None if rwork is None else rwork.data_ptr()
     # latency-sized rounds are faster as ONE kernel (measured: the second
     # launch costs the tail what the shortcut saves the bulk)
     TWO_KERNELS_ABOVE = 32768
-    if fd:
-        Xp = torch.empty((npts, B, n), dtype=f64, device=dev)
-        dx = torch.empty((B, 2 * n if fd3 else n), dtype=f64, device=dev)
     stream = lib.stream(X0)
-    lib.call("blsq_init_batched", meth, B, n, X0.data_ptr(), lb.data_ptr(),
-             ub.data_ptr(), bstride, state.data_ptr(), istate.data_ptr(),
-             Xnew.data_ptr(), stream)
+    perm = None
+    if not padded:
+        parts = [(n, 0, B)]
+    else:
+        ch = cols.cpu().to(torch.int64)
+        order = torch.argsort(ch, stable=True)
+        vals, cnt = torch.unique_consecutive(ch[order], return_counts=True)
+        perm = order.to(dev)
+        X0p = X0.index_select(0, perm)
+        if bstride:
+            lbp, ubp = lb.index_select(0, perm), ub.index_select(0, perm)
+        rowsp = None if rows is None else rows.index_select(0, perm)
+        parts, b0 = [], 0
+        for N, c in zip(vals.tolist(), cnt.tolist()):
+            parts.append((N, b0, c))
+            b0 += c
+    # count[k, 2] = problems of segment k still running after the last round
+    # (written by the round kernel itself, blsq_round_batched `count`)
+    count = torch.zeros((len(parts), 4), dtype=torch.int32, device=dev)
+    segs = []
+    for k, (N, b0, Bk) in enumerate(parts):
+        g = _Segment()
+        g.N, g.b0 = N, b0
+        if not padded:
+            g.x0, g.lb, g.ub, g.bs, g.rows = X0, lb, ub, bstride, rows
+        else:
+            sl = slice(b0, b0 + Bk)
+            g.x0 = X0p[sl, :N].contiguous()
+            g.x0pad = X0p[sl]                  # the held coordinates
+            g.lb = lbp[sl, :N].contiguous() if bstride else lb[:N]
+            g.ub = ubp[sl, :N].contiguous() if bstride else ub[:N]
+            g.bs = N if bstride else 0
+            g.rows = None if rows is None else rowsp[sl].contiguous()
+            g.perm = perm[sl]
+        g.lay = lib.state_layout(meth, N)
+        g.S = g.lay["size"]
+        g.LS = lib.lin_record_size(N)
+        g.max_nfev = int(100 * N if max_nfev is None else max_nfev)    # trf.py:234-235
+        g.npts = 2 * N if fd3 else N           # callback calls per FD Jacobian
+        g.state = torch.zeros((Bk, g.S), dtype=f64, device=dev)
+        g.istate = torch.zeros((Bk, L.ISTATE_SIZE), dtype=torch.int32, device=dev)
+        g.Xnew = torch.empty((Bk, N), dtype=f64, device=dev)
+        # dogbox evaluates J at the bound-snapped trial (dogbox.py:256-261)
+        g.Xjac = torch.empty((Bk, N), dtype=f64, device=dev) if method == "dogbox" \
+            else None
+        g.lin = torch.empty((Bk, g.LS), dtype=f64, device=dev)
+        g.count = count[k]
+        # TRF: worklist of the problems that leave the Gauss-Newton shortcut
+        # (blsq_round_batched `work`)
+        g.rwork = torch.empty(Bk + 1, dtype=torch.int32, device=dev) \
+            if method == "trf" else None
+        if fd:
+            g.Xp = torch.empty((g.npts, Bk, N), dtype=f64, device=dev)
+            g.dx = torch.empty((Bk, 2 * N if fd3 else N), dtype=f64, device=dev)
+        g.A, g.idx, g.idx32 = Bk, None, None   # idx: int64 for torch gathers
+        g.pong, g.flip, g.cwork = None, 0, None
+        lib.call("blsq_init_batched", meth, Bk, N, g.x0.data_ptr(), g.lb.data_ptr(),
+                 g.ub.data_ptr(), g.bs, g.state.data_ptr(), g.istate.data_ptr(),
+                 g.Xnew.data_ptr(), stream)
+        segs.append(g)
+    max_nfev = max(g.max_nfev for g in segs)
+    if padded:
+        # the padded callback batches, slots in segment order
+        Xcb = torch.empty((B, n), dtype=f64, device=dev)
+        Xjcb = torch.empty((B, n), dtype=f64, device=dev) if method == "dogbox" else None
+        if fd:
+            Xpcb = torch.empty((2 * n if fd3 else n, B, n), dtype=f64, device=dev)
+    gid = perm              # the callbacks' idx: original ids in slot order
 
-    # optional instrumentation (bench.py): CUDA events around every stage
+    # optional instrumentation (bench.py): CUDA events around every stage;
+    # a ragged-parameter batch keeps the linearise / round events per
+    # segment, under timers["segments"][N]
     def tick():
         if timers is None or not X0.is_cuda:
             return None
@@ -231,20 +295,20 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
         e.record()
         return e
 
-    def tock(kind, e0, running):
+    def tock(kind, e0, running, g=None):
         if e0 is None:
             return
         e1 = torch.cuda.Event(enable_timing=True)
         e1.record()
-        timers.setdefault(kind, []).append((e0, e1, running))
-    if timers is not None:
-        timers["shape"] = (n, None, LS, S)
+        if g is None:
+            timers.setdefault(kind, []).append((e0, e1, running))
+        else:
+            timers.setdefault("segments", {}).setdefault(g.N, {}).setdefault(
+                kind, []).append((e0, e1, g.A))
+    if timers is not None and not padded:
+        timers["shape"] = (n, None, segs[0].LS, segs[0].S)
     nrun = B
 
-    idx = None          # int64 for torch gathers
-    idx32 = None        # int32 copy handed to the kernels
-    pong, flip, cwork = None, 0, None
-    A = B
     first = 1
     m = None
     rounds = 0
@@ -252,46 +316,92 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
 
     # the dense entry points unless the batch is ragged (same kernels as
     # before for a dense batch, bit for bit)
-    def lin_call(*a):
-        if rows is None:
+    def lin_call(g, *a):
+        if padded:
+            lib.call("blsq_linearise_batched_ld", *a[:4], n, *a[4:])
+        elif g.rows is None:
             lib.call("blsq_linearise_batched", *a[:-2], a[-1])
         else:
             lib.call("blsq_linearise_batched_rows", *a)
 
-    def round_call(*a):
-        if rows is None:
+    def round_call(g, *a):
+        if g.rows is None:
             lib.call("blsq_round_batched", *a[:-2], a[-1])
         else:
             lib.call("blsq_round_batched_rows", *a)
 
-    def one_round(A, idx, idx32, first, nrun, off=0, count_here=True):
-        """Callbacks + linearise + round for the A compacted slots (or, in the
-        streaming prologue, for the A problems starting at problem `off`)."""
+    def pad(out, fdm, pick, counted=True):
+        """blsq_pad_points: the active points of every segment (pick(g) ->
+        (X, Xp or None)) into the padded batch `out`."""
+        nonlocal launches
+        live = [g for g in segs if g.A > 0]
+        tab = (L.PadSegment * len(live))()
+        s0 = 0
+        for i, g in enumerate(live):
+            X, Xp = pick(g)
+            tab[i] = L.PadSegment(s0, g.A, g.N, None if g.idx32 is None else g.idx32.data_ptr(),
+                                  g.x0pad.data_ptr(), X.data_ptr(),
+                                  None if Xp is None else Xp.data_ptr())
+            s0 += g.A
+        lib.call("blsq_pad_points", len(live), C.cast(tab, C.c_void_p), s0, n, fdm,
+                 out.data_ptr(), lib.stream(X0))
+        launches += counted
+
+    def one_round(first, nrun, pro=None, count_here=True):
+        """Callbacks + linearise + round for the active slots of every segment
+        (or, in the streaming prologue, pro = (off, A): for the A problems
+        starting at problem `off` of the one segment of a dense batch)."""
         nonlocal m, launches
         stream = lib.stream(X0)            # the capture stream inside a graph
-        Xa = Xnew[off:off + A]
-        Xj = Xa if (Xjac is None or first) else Xjac[off:off + A]
-        if idx is None and (off or A != B):
-            idx = slice(off, off + A)
-        # base pointers of this range of problems
-        p_ist = istate.data_ptr() + off * L.ISTATE_SIZE * 4
-        p_lin = lin.data_ptr() + off * LS * 8
-        p_st = state.data_ptr() + off * S * 8
-        p_x0 = X0.data_ptr() + off * n * 8
-        p_lb = lb.data_ptr() + off * bstride * 8
-        p_ub = ub.data_ptr() + off * bstride * 8
-        p_xn = Xnew.data_ptr() + off * n * 8
-        p_xj = None if Xjac is None else Xjac.data_ptr() + off * n * 8
-        # rows is indexed by problem id like istate: shifted the same way
-        p_rows = None if rows is None else rows.data_ptr() + off * 4
-        ip = None if idx32 is None else idx32.data_ptr()
+        off = 0
+        if pro is not None:
+            off, A = pro
+            live = [(segs[0], A)]
+        else:
+            live = [(g, g.A) for g in segs if g.A > 0]
+            A = sum(a for _, a in live)
+
+        def xj(g):                         # the points J is evaluated at
+            return g.Xnew if (g.Xjac is None or first) else g.Xjac
+        if padded:
+            idx = gid
+            Xa = Xcb[:A]
+            pad(Xa, 0, lambda g: (g.Xnew, None))
+            Xj = Xa
+            if Xjcb is not None and not first:
+                Xj = Xjcb[:A]
+                pad(Xj, 0, lambda g: (g.Xjac, None))
+        else:
+            g = segs[0]
+            Xa = g.Xnew[off:off + A]
+            Xj = Xa if (g.Xjac is None or first) else g.Xjac[off:off + A]
+            idx = g.idx
+            if idx is None and (off or A != B):
+                idx = slice(off, off + A)
+
+        # base pointers of this range of problems of each segment
+        def ptrs(g):
+            return dict(
+                ist=g.istate.data_ptr() + off * L.ISTATE_SIZE * 4,
+                lin=g.lin.data_ptr() + off * g.LS * 8,
+                st=g.state.data_ptr() + off * g.S * 8,
+                x0=g.x0.data_ptr() + off * g.N * 8,
+                lb=g.lb.data_ptr() + off * g.bs * 8,
+                ub=g.ub.data_ptr() + off * g.bs * 8,
+                xn=g.Xnew.data_ptr() + off * g.N * 8,
+                xj=None if g.Xjac is None else g.Xjac.data_ptr() + off * g.N * 8,
+                # rows is indexed by problem id like istate: shifted the same way
+                rows=None if g.rows is None else g.rows.data_ptr() + off * 4,
+                ip=None if g.idx32 is None else g.idx32.data_ptr())
+        P = [ptrs(g) for g, _ in live]
         # a model compiled into the linearisation kernel replaces the two
         # callbacks and blsq_linearise_batched of this round by one launch
         cbs = getattr(fun, "__self__", None)
         mm = None
-        if not fd and Xjac is None and rows is None and hasattr(cbs, "lin"):
+        if not padded and not fd and segs[0].Xjac is None and segs[0].rows is None \
+                and hasattr(cbs, "lin"):
             t0 = tick()
-            mm = cbs.lin(Xa, idx32, off, A, p_ist, p_lin, stream)
+            mm = cbs.lin(Xa, segs[0].idx32, off, A, P[0]["ist"], P[0]["lin"], stream)
             if mm is not None:
                 m = mm
                 launches += 1
@@ -319,45 +429,69 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
                     raise RuntimeError(
                         "Inconsistent dimensions between the returns of `fun` "
                         "and `jac` on the first iteration.")
+                # aligned for width n is aligned for every segment's N
+                # (lin_ld_width(N, n) divides n)
                 J = L.aligned(J.contiguous(), 32 if n % 4 == 0 else (16 if n % 2 == 0 else 8))
                 tock("callbacks", t0, nrun)
-                t0 = tick()
-                lin_call(A, ip, m, n, F.data_ptr(), J.data_ptr(), None, None, 0,
-                         p_ist, p_lin, p_rows, stream)
-                tock("linearise", t0, nrun)
+                s0 = 0
+                for (g, a), p in zip(live, P):
+                    t0 = tick()
+                    lin_call(g, a, p["ip"], m, g.N, F.data_ptr() + s0 * m * 8,
+                             J.data_ptr() + s0 * m * n * 8, None, None, 0,
+                             p["ist"], p["lin"], p["rows"], stream)
+                    tock("linearise", t0, nrun, g if padded else None)
+                    s0 += a
             else:
-                Xpa = Xp.view(-1)[: npts * A * n].view(npts, A, n)
-                lib.call("blsq_fd3_points" if fd3 else "blsq_fd2_points", A, ip, n,
-                         Xj.data_ptr(), p_lb, p_ub, bstride, rel,
-                         Xpa.data_ptr(), dx.data_ptr(), stream)
-                launches += 1
+                for (g, a), p in zip(live, P):
+                    Xpa = g.Xp.view(-1)[: g.npts * a * g.N].view(g.npts, a, g.N)
+                    lib.call("blsq_fd3_points" if fd3 else "blsq_fd2_points", a, p["ip"],
+                             g.N, (xj(g) if padded else Xj).data_ptr(),
+                             p["lb"], p["ub"], g.bs, rel, Xpa.data_ptr(), g.dx.data_ptr(),
+                             stream)
+                    launches += 1
+                npts = 2 * n if fd3 else n
+                if padded:
+                    Xpa = Xpcb.view(-1)[: npts * A * n].view(npts, A, n)
+                    pad(Xpa, 2 if fd3 else 1, lambda g: (xj(g), g.Xp))
                 Fp = []
                 for i in range(npts):
                     Fi = _as_f64(fun(Xpa[i], idx), X0, "fun").contiguous()
                     if Fi.shape != F.shape:
                         raise RuntimeError("`fun` changed its output shape")
                     Fp.append(Fi)
-                plist = (C.c_void_p * npts)(*[t.data_ptr() for t in Fp])
                 tock("callbacks", t0, nrun)
-                t0 = tick()
-                lin_call(A, ip, m, n, F.data_ptr(), None,
-                         C.cast(plist, C.c_void_p), dx.data_ptr(), 2 if fd3 else 1,
-                         p_ist, p_lin, p_rows, stream)
-                tock("linearise", t0, nrun)
-        t0 = tick()
-        round_call(meth, A, ip, m, n, p_lin,
-                   p_x0, p_lb, p_ub, bstride, sc_ptr,
-                   float(ftol), float(xtol), float(gtol), max_nfev, first,
-                   p_st, p_ist, p_xn, p_xj,
-                   rwork_ptr if A >= TWO_KERNELS_ABOVE else None,
-                   count.data_ptr() if count_here else None, p_rows, stream)
-        tock("round", t0, nrun)
-        if timers is not None:
-            timers["shape"] = (n, m, LS, S)
-        launches += (2 if (rwork is None or A < TWO_KERNELS_ABOVE) else 3) - \
-            (1 if mm is not None else 0)
+                s0 = 0
+                for (g, a), p in zip(live, P):
+                    # segment g reads its slots of the batches of its own N
+                    # coordinates; the other batches are not read
+                    plist = (C.c_void_p * g.npts)(*[t.data_ptr() + s0 * m * 8
+                                                    for t in Fp[:g.npts]])
+                    t0 = tick()
+                    lin_call(g, a, p["ip"], m, g.N, F.data_ptr() + s0 * m * 8, None,
+                             C.cast(plist, C.c_void_p), g.dx.data_ptr(), 2 if fd3 else 1,
+                             p["ist"], p["lin"], p["rows"], stream)
+                    tock("linearise", t0, nrun, g if padded else None)
+                    s0 += a
+        for (g, a), p in zip(live, P):
+            t0 = tick()
+            round_call(g, meth, a, p["ip"], m, g.N, p["lin"],
+                       p["x0"], p["lb"], p["ub"], g.bs, sc_ptr,
+                       float(ftol), float(xtol), float(gtol), g.max_nfev, first,
+                       p["st"], p["ist"], p["xn"], p["xj"],
+                       g.rwork.data_ptr() if (g.rwork is not None and a >= TWO_KERNELS_ABOVE)
+                       else None,
+                       g.count.data_ptr() if count_here else None, p["rows"], stream)
+            tock("round", t0, nrun, g if padded else None)
+            launches += 2 if (g.rwork is None or a < TWO_KERNELS_ABOVE) else 3
+        if timers is not None and not padded:
+            timers["shape"] = (n, m, segs[0].LS, segs[0].S)
+        launches -= 1 if mm is not None else 0
 
-    def graph_tail(A, idx, idx32, nrun):
+    def running():
+        """Problems still running per segment: the one host sync."""
+        return count.cpu()[:, 2].tolist()
+
+    def graph_tail(nrun):
         """The latency-sized tail of the batch (A <= tail_below slots, often a
         hundred more rounds for the slowest problems): GRAPH_ROUNDS rounds +
         the status count are captured ONCE into a CUDA graph and replayed, so
@@ -367,7 +501,7 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
         run, or None if the callbacks cannot be captured (host syncs,
         data-dependent shapes): the caller then carries on eagerly."""
         nonlocal launches
-        one_round(A, idx, idx32, 0, nrun)       # eager: errors surface here
+        one_round(0, nrun)                     # eager: errors surface here
         r = 1
         l1 = launches
         # torch.cuda.graph() synchronises the device and flushes the caching
@@ -390,7 +524,7 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
                                 capture_error_mode="thread_local")
                 try:
                     for _ in range(GRAPH_ROUNDS):
-                        one_round(A, idx, idx32, 0, nrun)
+                        one_round(0, nrun)
                 finally:
                     g.capture_end()
             cur.wait_stream(side)
@@ -417,7 +551,7 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
             g.replay()
             launches += per_replay
             r += GRAPH_ROUNDS
-            if int(count[2].item()) == 0 or rounds + r > max_nfev + 1:
+            if sum(running()) == 0 or rounds + r > max_nfev + 1:
                 return r, True
 
     if graph_tail_rounds is None:                  # BLSQ_GRAPH_TAIL=0 turns it off
@@ -426,6 +560,13 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
                  and timers is None
                  and _cb_key(fun, jac) not in _NOT_CAPTURABLE)
     GRAPH_ROUNDS = int(graph_tail_rounds)
+    if prologue and padded:
+        # the streaming prologue runs the problems in their original order,
+        # not in segments: wait for every copy and start in lock step
+        for _, _, ev in prologue:
+            if ev is not None:
+                torch.cuda.current_stream(dev).wait_event(ev)
+        prologue = None
     if prologue:
         # streaming start: the per-problem data arrives from the host in
         # chunks; each chunk runs its first rounds alone while the next one is
@@ -440,57 +581,88 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
             if ev is not None:
                 torch.cuda.current_stream(dev).wait_event(ev)
             for r in range(K):
-                one_round(c1 - c0, None, None, 1 if r == 0 else 0, c1 - c0, off=c0,
-                          count_here=False)
+                one_round(1 if r == 0 else 0, c1 - c0, pro=(c0, c1 - c0), count_here=False)
         first = 0
         rounds = K
 
-    def compact(A, idx32, nrun):
-        """Ordered compaction on the device (3 small launches) into the other
-        half of a ping-pong pair; the nrun problems still running (the round
-        kernel's count) fill its first slots."""
-        nonlocal pong, flip, cwork, launches, Xnew, Xjac
-        if pong is None:
-            pong = [dict(X=torch.empty_like(Xnew),
-                         J=None if Xjac is None else torch.empty_like(Xjac),
-                         i32=torch.empty(A, dtype=torch.int32, device=dev),
-                         i64=torch.empty(A, dtype=torch.int64, device=dev)),
-                    dict(X=Xnew, J=Xjac,
-                         i32=torch.empty(A, dtype=torch.int32, device=dev),
-                         i64=torch.empty(A, dtype=torch.int64, device=dev))]
-            cwork = torch.empty(int(lib._dll.blsq_compact_work_size(A)),
-                                dtype=torch.int32, device=dev)
-        o = pong[flip]
-        flip ^= 1
-        lib.call("blsq_compact_batched", A,
-                 None if idx32 is None else idx32.data_ptr(),
-                 istate.data_ptr(), n, Xnew.data_ptr(),
-                 None if Xjac is None else Xjac.data_ptr(),
+    def compact(g, nrun):
+        """Ordered compaction of segment g on the device (3 small launches)
+        into the other half of a ping-pong pair; the nrun problems still
+        running (the round kernel's count) fill its first slots."""
+        nonlocal launches
+        if g.pong is None:
+            g.pong = [dict(X=torch.empty_like(g.Xnew),
+                           J=None if g.Xjac is None else torch.empty_like(g.Xjac),
+                           i32=torch.empty(g.A, dtype=torch.int32, device=dev),
+                           i64=torch.empty(g.A, dtype=torch.int64, device=dev)),
+                      dict(X=g.Xnew, J=g.Xjac,
+                           i32=torch.empty(g.A, dtype=torch.int32, device=dev),
+                           i64=torch.empty(g.A, dtype=torch.int64, device=dev))]
+            g.cwork = torch.empty(int(lib._dll.blsq_compact_work_size(g.A)),
+                                  dtype=torch.int32, device=dev)
+        o = g.pong[g.flip]
+        g.flip ^= 1
+        lib.call("blsq_compact_batched", g.A,
+                 None if g.idx32 is None else g.idx32.data_ptr(),
+                 g.istate.data_ptr(), g.N, g.Xnew.data_ptr(),
+                 None if g.Xjac is None else g.Xjac.data_ptr(),
                  o["i32"].data_ptr(), o["i64"].data_ptr(),
                  o["X"].data_ptr(),
-                 None if Xjac is None else o["J"].data_ptr(),
-                 cwork.data_ptr(), lib.stream(X0))
+                 None if g.Xjac is None else o["J"].data_ptr(),
+                 g.cwork.data_ptr(), lib.stream(X0))
         launches += 3
-        Xnew, Xjac = o["X"], o["J"]
-        return nrun, o["i64"][:nrun], o["i32"][:nrun]
+        g.Xnew, g.Xjac = o["X"], o["J"]
+        g.A, g.idx, g.idx32 = nrun, o["i64"][:nrun], o["i32"][:nrun]
 
+    def trace_view():
+        """trace(rounds, idx, X, state, istate) arguments: the next trial
+        points of the active slots in callback order, with istate indexed by
+        problem id (state: the segments' records of a ragged-parameter batch)."""
+        if not padded:
+            g = segs[0]
+            return g.idx, g.Xnew[:g.A], g.state, g.istate
+        X = torch.empty((A, n), dtype=f64, device=dev)
+        pad(X, 0, lambda g: (g.Xnew, None), counted=False)
+        ist = torch.empty((B, L.ISTATE_SIZE), dtype=torch.int32, device=dev)
+        ist[perm] = torch.cat([g.istate for g in segs])
+        return gid, X, [g.state for g in segs], ist
+
+    A = B
     while A > 0:
-        one_round(A, idx, idx32, first, nrun)
+        one_round(first, nrun)
         first = 0
         rounds += 1
         if trace is not None:
-            trace(rounds, idx, Xnew[:A], state, istate)
+            trace(rounds, *trace_view())
         # host look at the status flags: every second round while the rounds
         # are bandwidth-sized, every 4th once they are launch-latency sized
         every = check_every if A > tail_below else max(check_every, 4)
         if rounds % every == 0 or rounds >= max_nfev:
-            nrun = int(count[2].item())               # the one host sync
+            nrs = running()                           # the one host sync
+            nrun = sum(nrs)
             if nrun == 0:
                 break
-            if nrun <= compact_below * A:
-                A, idx, idx32 = compact(A, idx32, nrun)
+            moved = []
+            for g, nr in zip(segs, nrs):
+                if g.A and nr <= compact_below * g.A:
+                    moved.append((g, int(lib._dll.blsq_compact_work_size(g.A)) - 1))
+                    compact(g, nr)
+            if moved and padded:
+                # the round kernel counts before the deferred TRF pass, which
+                # can still finish problems: the slots past the survivors
+                # would hold stale ids, and a segment's ids only index its own
+                # problems.  The compaction's own survivor counts, one sync.
+                surv = torch.stack([g.cwork[w] for g, w in moved]).cpu().tolist()
+                for (g, _), s in zip(moved, surv):
+                    g.A, g.idx, g.idx32 = s, g.idx[:s], g.idx32[:s]
+                    if s == 0:
+                        g.count.zero_()       # no longer launched: not running
+            A = sum(g.A for g in segs)
+            if moved and padded:
+                gid = torch.cat([g.perm if g.idx is None else g.perm.index_select(0, g.idx)
+                                 for g in segs if g.A > 0])
             if use_graph and A <= tail_below:
-                r, done = graph_tail(A, idx, idx32, nrun)
+                r, done = graph_tail(nrun)
                 rounds += r
                 if done:
                     break
@@ -498,7 +670,16 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
         if rounds > max_nfev + 1:                     # cannot happen
             raise RuntimeError("batched driver failed to terminate")
 
-    status = istate[:, 0].to(torch.int64)
+    if padded:
+        inv = torch.empty_like(perm)
+        inv[perm] = torch.arange(B, device=dev)
+
+    def gather(t):                                    # segment order -> problem order
+        return t if not padded else t.index_select(0, inv)
+
+    def field(f):
+        return gather(f(segs[0]) if not padded else torch.cat([f(g) for g in segs]))
+    status = field(lambda g: g.istate[:, 0].to(torch.int64))
     bad = status < L.STATUS_RUNNING
     if bool(bad.any().item()):
         # trust_region.py:28-35 raises these from inside trf.  One problem:
@@ -520,25 +701,42 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
             % (which.numel(), B, L.STATUS_ERR_TR_ZERO, L.STATUS_ERR_TR_OUTSIDE,
                which[:8].tolist()), RuntimeWarning)
 
-    x = state[:, lay["x"]:lay["x"] + n].contiguous()
-    if method == "trf":
-        # trf.py:257,354: find_active_constraints(x, lb, ub, rtol=xtol)
-        mask = lib.find_active_constraints(x, lb, ub, xtol)
-    else:
-        mask = torch.empty((B, n), dtype=torch.int64, device=dev)
-        lib.call("blsq_dogbox_on_bound", B, n, istate.data_ptr(),
-                 mask.data_ptr(), stream)
-    cov = None
-    if x_covariance:
-        # (J^T J)^-1 at the returned x from the triangle the solve holds
-        cov = torch.empty((B, n, n), dtype=f64, device=dev)
-        lib.call("blsq_covariance", B, n, state.data_ptr(), S, lay["R"], 1,
-                 cov.data_ptr(), stream)
+    # per segment; a ragged-parameter batch pads x with x0, active_mask and
+    # x_covariance with zeros
+    if padded:
+        x = X0p.clone()
+        mask = torch.zeros((B, n), dtype=torch.int64, device=dev)
+        cov = torch.zeros((B, n, n), dtype=f64, device=dev) if x_covariance else None
+    for g in segs:
+        N, Bk, b1 = g.N, g.state.shape[0], g.b0 + g.state.shape[0]
+        xg = g.state[:, g.lay["x"]:g.lay["x"] + N].contiguous()
+        if method == "trf":
+            # trf.py:257,354: find_active_constraints(x, lb, ub, rtol=xtol)
+            mg = lib.find_active_constraints(xg, g.lb, g.ub, xtol)
+        else:
+            mg = torch.empty((Bk, N), dtype=torch.int64, device=dev)
+            lib.call("blsq_dogbox_on_bound", Bk, N, g.istate.data_ptr(),
+                     mg.data_ptr(), stream)
+        cg = None
+        if x_covariance:
+            # (J^T J)^-1 at the returned x from the triangle the solve holds
+            cg = torch.empty((Bk, N, N), dtype=f64, device=dev)
+            lib.call("blsq_covariance", Bk, N, g.state.data_ptr(), g.S, g.lay["R"], 1,
+                     cg.data_ptr(), stream)
+        if not padded:
+            x, mask, cov = xg, mg, cg
+        else:
+            x[g.b0:b1, :N] = xg
+            mask[g.b0:b1, :N] = mg
+            if x_covariance:
+                cov[g.b0:b1, :N, :N] = cg
     return dict(
-        x_covariance=cov,
-        x=x, obj_value=state[:, lay["obj"]].clone(),
-        optimality=state[:, lay["gnorm"]].clone(), active_mask=mask,
-        nfev=istate[:, 1].to(torch.int64), njev=istate[:, 2].to(torch.int64),
+        x_covariance=None if cov is None else gather(cov),
+        x=gather(x), obj_value=field(lambda g: g.state[:, g.lay["obj"]].clone()),
+        optimality=field(lambda g: g.state[:, g.lay["gnorm"]].clone()),
+        active_mask=gather(mask),
+        nfev=field(lambda g: g.istate[:, 1].to(torch.int64)),
+        njev=field(lambda g: g.istate[:, 2].to(torch.int64)),
         status=status, m=m, rounds=rounds, kernel_launches=launches)
 
 

@@ -171,6 +171,35 @@ compact_scatter_kernel(int64_t A, const int32_t* __restrict__ idx,
     }
 }
 
+// ---- padded trial batches of a ragged-parameter batch (blsq_pad_points) ------
+struct PadTable {
+    blsq_pad_segment seg[BLSQ_MAX_BATCHED_N];
+    int nseg;
+};
+
+// one thread per (batch p, slot, coordinate k) of out (P, A, n)
+__global__ void pad_points_kernel(PadTable tab, int64_t A, int n, int fd,
+                                  double* __restrict__ out) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int64_t P = fd ? (int64_t)fd * n : 1;
+    if (t >= P * A * n) return;
+    const int k = (int)(t % n);
+    const int64_t slot = (t / n) % A;
+    const int p = (int)(t / ((int64_t)n * A));
+    int j = 0;
+    while (j + 1 < tab.nseg && slot >= tab.seg[j + 1].off) j++;
+    const blsq_pad_segment& g = tab.seg[j];
+    const int64_t s = slot - g.off;
+    double v;
+    if (k >= g.n)
+        v = g.x0[(g.idx ? (int64_t)g.idx[s] : s) * n + k];      // held fixed
+    else if (fd && p < fd * g.n)
+        v = g.Xp[((int64_t)p * g.A + s) * g.n + k];             // its own FD point
+    else
+        v = g.X[s * g.n + k];
+    out[t] = v;
+}
+
 }  // namespace
 
 #ifdef BLSQ_ONLY_N46      /* quick builds for tools/build_variants.sh */
@@ -286,8 +315,7 @@ int blsq_linearise_batched_rows(int64_t A, const int32_t* idx, int m, int n,
     if (jac_mode == 0 && !J) return BLSQ_E_BADARG;
     // lin_kernel loads the rows of J with 256-bit (n % 4 == 0) or 128-bit
     // (n = 2, 6, 10, 14) vector loads: a misaligned J would fault the device
-    if (jac_mode == 0 && (uintptr_t)J % (n % 4 == 0 ? 32 : (n % 2 == 0 ? 16 : 8)))
-        return BLSQ_E_BADARG;
+    if (jac_mode == 0 && (uintptr_t)J % (8 * lin_ld_width(n, n))) return BLSQ_E_BADARG;
     if (jac_mode != 0 && (!dx || !Fp_host)) return BLSQ_E_BADARG;
     if (jac_mode != 0 && n >= 1 && n <= BLSQ_MAX_BATCHED_N)
         for (int j = 0; j < jac_mode * n; j++)
@@ -307,6 +335,53 @@ int blsq_linearise_batched(int64_t A, const int32_t* idx, int m, int n,
                            void* stream) {
     return blsq_linearise_batched_rows(A, idx, m, n, F, J, Fp_host, dx, jac_mode, istate,
                                        lin, nullptr, stream);
+}
+
+int blsq_linearise_batched_ld(int64_t A, const int32_t* idx, int m, int n, int ldj,
+                              const double* F, const double* J,
+                              const double* const* Fp_host, const double* dx,
+                              int jac_mode, const int32_t* istate, double* lin,
+                              const int32_t* rows, void* stream) {
+    if (ldj < n) return BLSQ_E_BADARG;
+    if (ldj == n || jac_mode != 0)
+        return blsq_linearise_batched_rows(A, idx, m, n, F, J, Fp_host, dx, jac_mode, istate,
+                                           lin, rows, stream);
+    if (A < 0 || m < 1 || !F || !J || !istate || !lin) return BLSQ_E_BADARG;
+    // a row of J starts only as aligned as ldj * 8 bytes allows: the vector
+    // width follows from both n and ldj, and J must be aligned to it
+    if ((uintptr_t)J % (8 * lin_ld_width(n, ldj))) return BLSQ_E_BADARG;
+    if (A == 0) return 0;
+#ifdef BLSQ_ONLY_N46
+    return BLSQ_E_UNSUPPORTED;
+#else
+    BLSQ_DISPATCH_N(n, {
+        return ld_launch_lin<N_>(A, idx, m, ldj, F, J, istate, lin, rows, (cudaStream_t)stream);
+    });
+    return 0;
+#endif
+}
+
+int blsq_pad_points(int nseg, const blsq_pad_segment* seg_host, int64_t A, int n, int fd,
+                    double* out, void* stream) {
+    if (nseg < 1 || nseg > BLSQ_MAX_BATCHED_N || !seg_host || !out || A < 0) return BLSQ_E_BADARG;
+    if (n < 1 || n > BLSQ_MAX_BATCHED_N || fd < 0 || fd > 2) return BLSQ_E_BADARG;
+    PadTable tab;
+    tab.nseg = nseg;
+    int64_t off = 0;
+    for (int j = 0; j < nseg; j++) {
+        const blsq_pad_segment& g = seg_host[j];
+        if (g.off != off || g.A < 0 || g.n < 1 || g.n > n) return BLSQ_E_BADARG;
+        if (g.A > 0 && (!g.x0 || !g.X || (fd && !g.Xp))) return BLSQ_E_BADARG;
+        tab.seg[j] = g;
+        off += g.A;
+    }
+    if (off != A) return BLSQ_E_BADARG;
+    if (A == 0) return 0;
+    const int64_t total = (fd ? (int64_t)fd * n : 1) * A * n;
+    pad_points_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+        tab, A, n, fd, out);
+    BLSQ_LAUNCH_CHECK();
+    return 0;
 }
 
 int blsq_round_batched_rows(int method, int64_t A, const int32_t* idx, int m, int n,

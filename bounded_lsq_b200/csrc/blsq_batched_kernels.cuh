@@ -335,6 +335,13 @@ int launch_round(int method, int64_t A, const int32_t* idx, const double* lin,
 
 }  // namespace
 
+// lin_kernel for a Jacobian padded to ldj > N columns (blsq_linearise_batched_ld),
+// defined in blsq_batched_ld.cu, one object per N
+template <int N>
+int ld_launch_lin(int64_t A, const int32_t* idx, int m, int ldj, const double* F,
+                  const double* J, const int32_t* istate, double* lin,
+                  const int32_t* rows, cudaStream_t s);
+
 // the instances for N = 9..16, defined in blsq_batched_wide.cu
 template <int N>
 int wide_launch_lin(int64_t A, const int32_t* idx, int m, const double* F,

@@ -100,6 +100,13 @@ __device__ __forceinline__ double div_rn(double a, double b, double y) {
 
 template <int N> struct PtrList { const double* p[2 * N]; };   // 2 per coordinate (3-point)
 
+// Doubles per vector load of a row of J with n columns at row stride ldj: a
+// row starts only as aligned as ldj * 8 bytes allows (J itself aligned to as
+// many).  ldj == n gives the dense widths: 4 for n % 4 == 0, 2 for even n.
+__host__ __device__ constexpr int lin_ld_width(int n, int ldj) {
+    return (n % 4 == 0 && ldj % 4 == 0) ? 4 : ((n % 2 == 0 && ldj % 2 == 0) ? 2 : 1);
+}
+
 // One group of G lanes (G = 8, 16 or 32) per problem; row (base + s*G + lane)
 // of the current chunk sits in a[s][*] of that lane.
 // MODE 0: analytic J (A, m, n).  MODE 1: 2-point differences, Fpert.p[i] is
@@ -117,13 +124,24 @@ template <int N> struct PtrList { const double* p[2 * N]; };   // 2 per coordina
 // its first rows[pid] residuals with the same lane group.  MULTI folds chunks
 // only up to the problem's own count.  The dense path (ROWS = false) is a
 // separate instance and compiles to the code it had before.
-template <int N, int G, int MODE, bool MULTI, class MODEL = NoModel, bool ROWS = false>
+// LDW > 0 (MODE 0 with ROWS only): J is the (A, m, ldj) output of a batch
+// padded to ldj > N parameters (least_squares_batched `cols`); the first N
+// columns of each row are read with LDW-double vector loads
+// (lin_ld_width(N, ldj)) and the others never are.  rows may be null there
+// (every problem has m rows).  Otherwise the same instructions as the
+// ROWS instance, so the record is that of a dense (A, m, N) Jacobian.
+template <int N, int G, int MODE, bool MULTI, class MODEL = NoModel, bool ROWS = false,
+          int LDW = 0>
 __global__ void __launch_bounds__(BLSQ_LIN_THREADS, LinCfg<N>::MINB)
 lin_kernel(int64_t A, const int32_t* __restrict__ idx, int m,
            const double* __restrict__ F, const double* __restrict__ J,
            PtrList<N> Fpert, const double* __restrict__ dx,
            const int32_t* __restrict__ istate, double* __restrict__ lin,
-           MODEL mdl = MODEL(), const int32_t* __restrict__ rows = nullptr) {
+           MODEL mdl = MODEL(), const int32_t* __restrict__ rows = nullptr, int ldj = 0) {
+    static_assert(LDW == 0 || (MODE == 0 && ROWS && N % LDW == 0), "LDW");
+    // doubles per vector load of a row of J, and the row stride of J
+    constexpr int VW = LDW ? LDW : (N % 4 == 0 ? 4 : (N % 2 == 0 ? 2 : 1));
+    const int rs = LDW ? ldj : N;
     constexpr int RPL = LinCfg<N>::RPL;
     constexpr int C = N + 1;                      // columns of [J | f]
     constexpr int AR = MULTI ? RPL + 1 : RPL;     // + carried row of the triangle
@@ -142,12 +160,12 @@ lin_kernel(int64_t A, const int32_t* __restrict__ idx, int m,
     // rows of this problem (ROWS; MULTI: G = 32, so the count is warp-uniform)
     int mp = m;
     if (ROWS && valid) {
-        const int r = rows[pid];
+        const int r = (LDW && !rows) ? m : rows[pid];
         mp = r < 0 ? 0 : (r > m ? m : r);
     }
 
     const double* Fp = (MODE == 3) ? nullptr : F + slot * (int64_t)m;
-    const double* Jp = (MODE == 0) ? J + slot * (int64_t)m * N : nullptr;
+    const double* Jp = (MODE == 0) ? J + slot * (int64_t)m * rs : nullptr;
     double* out = lin + slot * (int64_t)L::SIZE;
 
     double a[AR][C];
@@ -191,8 +209,8 @@ lin_kernel(int64_t A, const int32_t* __restrict__ idx, int m,
                     mdl.template row<N>(slot, pid, row, a[s]);
                 } else if (ok) {
                     if (MODE == 0) {
-                        const double* rp = Jp + (int64_t)row * N;
-                        if (N % 4 == 0) {
+                        const double* rp = Jp + (int64_t)row * rs;
+                        if (VW == 4) {
                             // 256-bit streaming loads: a whole 32-byte sector per
                             // instruction and lane (rows of 4 / 8 doubles)
 #pragma unroll
@@ -201,7 +219,7 @@ lin_kernel(int64_t A, const int32_t* __restrict__ idx, int m,
                                              : "=d"(a[s][j]), "=d"(a[s][j + 1]),
                                                "=d"(a[s][j + 2]), "=d"(a[s][j + 3])
                                              : "l"(rp + j));
-                        } else if (N % 2 == 0) {
+                        } else if (VW == 2) {
 #pragma unroll
                             for (int j = 0; j < N; j += 2) {
                                 double2 t = __ldcs(reinterpret_cast<const double2*>(rp + j));

@@ -94,21 +94,26 @@ def prepare_bounds(bounds, x0):
     return lb.contiguous(), ub.contiguous()
 
 
-def check_scaling(scaling, x0):
-    """least_squares.py:100-117 (shared across the batch: shape (n,))."""
+def check_scaling(scaling, x0, used=None):
+    """least_squares.py:100-117 (shared across the batch: shape (n,)).  used:
+    only the first `used` entries must be positive (ragged `cols`: the
+    entries past the largest count are never read)."""
     if isinstance(scaling, str) and scaling == 'jac':
         return scaling
     try:
         scaling = _to_f64(scaling, x0.device)
     except (ValueError, TypeError, RuntimeError):
         raise ValueError("`scaling` must be 'jac' or array-like with numbers.")
-    if bool(torch.any(scaling <= 0).item()):
-        raise ValueError("`scaling` must contain only positive values.")
     n = x0.shape[-1]
     if scaling.dim() == 0:
         scaling = scaling.expand(n)
+    if used is None:
+        if bool(torch.any(scaling <= 0).item()):
+            raise ValueError("`scaling` must contain only positive values.")
     if scaling.shape != (n,):
         raise ValueError("Inconsistent shapes between `scaling` and `x0`.")
+    if used is not None and bool(torch.any(scaling[:used] <= 0).item()):
+        raise ValueError("`scaling` must contain only positive values.")
     return scaling.contiguous()
 
 
@@ -141,7 +146,8 @@ def least_squares_batched(fun, x0, jac='2-point', bounds=(-float('inf'), float('
 
     ``options``: ``chunk`` (solve the batch that many problems at a time),
     ``x_covariance``, ``h2d_chunks`` / ``device`` (host inputs), ``rows``
-    (ragged batches, below), and the driver knobs of ``batched.solve_batched``.
+    and ``cols`` (ragged batches, below), and the driver knobs of
+    ``batched.solve_batched``.
 
     Ragged batches, ``options={'rows': rows}``: ``rows`` is an integer tensor of
     shape (B,), on the CPU or on the solve's device.  The callbacks keep
@@ -155,6 +161,30 @@ def least_squares_batched(fun, x0, jac='2-point', bounds=(-float('inf'), float('
     like the other per-problem data.  Not available with models compiled into
     the linearisation (``models.callbacks(..., 'inlined')``).  Without
     ``rows`` the solve is exactly the dense one.
+
+    Ragged parameter counts, ``options={'cols': cols}``: ``cols`` is an
+    integer tensor of shape (B,), on the CPU or on the solve's device, with
+    1 <= cols[b] <= n.  Problem b is solved as the reference solves the
+    problem made of its first cols[b] parameters: x0, bounds and scaling cut
+    to cols[b] entries, ``max_nfev=None`` meaning 100 * cols[b], and every
+    n-dependent decision (full-rank test, dogbox's rcond, the norms) taking
+    cols[b].  Its other coordinates are held fixed: in every X handed to
+    ``fun`` / ``jac`` (trial and finite-difference points) they are x0[b]
+    unchanged, so a callback may read them as fixed model parameters, and
+    ``res.x`` returns them unchanged.  Jacobian columns past cols[b] are never
+    read (they may hold anything, NaN included); bounds and scaling past
+    cols[b] are not checked.  ``active_mask`` is 0 and ``x_covariance`` has
+    zero rows and columns past cols[b].  The batch runs as one segment per
+    distinct count (at most 16), in lock step with one callback call per
+    round: the callbacks see the running problems segment by segment (the
+    stable sort of the problems by cols[b]), so per-problem data must be
+    passed as ``PerProblem`` (or read through the ids of the indexed
+    protocol).  ``cols`` works with ``rows``, ``chunk``, per-problem bounds,
+    the analytic and finite-difference Jacobians and ``x_covariance``.  Host
+    inputs are staged as without it, but the first round waits for every
+    copy: the streaming prologue runs the problems in their original order,
+    not segment by segment.  Not available with models compiled into the
+    linearisation.  Without ``cols`` the solve is exactly the dense one.
     """
     lib = _lib if _lib is not None else L.get_lib()
     _validate_common(method, bounds, jac)
@@ -169,9 +199,10 @@ def least_squares_batched(fun, x0, jac='2-point', bounds=(-float('inf'), float('
     guard = torch.cuda.device(target) if target is not None else \
         lib.device_guard(None)
     chunk = options.pop("chunk", None)
-    if options.get("rows") is not None and getattr(fun, "blsq_linearise", None) is not None:
-        raise ValueError("`rows` is not supported with a model compiled into the "
-                         "linearisation (models.callbacks(..., 'inlined')).")
+    for key in ("rows", "cols"):
+        if options.get(key) is not None and getattr(fun, "blsq_linearise", None) is not None:
+            raise ValueError(f"`{key}` is not supported with a model compiled into the "
+                             "linearisation (models.callbacks(..., 'inlined')).")
     with guard:
         if chunk is not None and isinstance(x0, torch.Tensor) and x0.dim() == 2 \
                 and x0.shape[0] > int(chunk) > 0:
@@ -193,6 +224,7 @@ def _least_squares_chunked(lib, chunk, fun, x0, jac, bounds, method, ftol, xtol,
     B = x0.shape[0]
     plan = None
     rows = options.pop("rows", None)
+    cols = options.pop("cols", None)
     if lib.requires_cuda and not x0.is_cuda:
         x0, args, kwargs, plan = _stage_host_inputs(x0, args, kwargs, options)
     else:
@@ -200,6 +232,8 @@ def _least_squares_chunked(lib, chunk, fun, x0, jac, bounds, method, ftol, xtol,
         options.pop("device", None)
     if rows is not None:
         rows = _check_rows(rows, B, x0.device)         # copied once, sliced per chunk
+    if cols is not None:
+        cols = _check_cols(cols, B, x0.shape[-1], x0.device)
 
     def part(v, c0, c1):
         if isinstance(v, PerProblem):
@@ -224,6 +258,8 @@ def _least_squares_chunked(lib, chunk, fun, x0, jac, bounds, method, ftol, xtol,
         opts = dict(options)
         if rows is not None:
             opts["rows"] = rows[c0:c1]
+        if cols is not None:
+            opts["cols"] = cols[c0:c1]
         outs.append(_least_squares_batched(
             lib, fun, x0[c0:c1], jac, (bound(bounds[0], c0, c1), bound(bounds[1], c0, c1)),
             method, ftol, xtol, gtol, max_nfev, scaling, diff_step,
@@ -251,11 +287,13 @@ def _least_squares_batched(lib, fun, x0, jac, bounds, method, ftol, xtol, gtol,
         # they are streamed to the device in chunks and the first rounds of
         # each chunk overlap the transfer of the next one
         x0, args, kwargs, plan = _stage_host_inputs(x0, args, kwargs, options)
-        if plan is not None and "trace" not in options:
+        if plan is not None and "trace" not in options and options.get("cols") is None:
             options["prologue"] = plan
         elif plan is not None:
-            # not streamed (the trace hook wants whole-batch rounds): the
-            # copies were queued on the side stream, wait for the last one
+            # not streamed (the trace hook wants whole-batch rounds; `cols`
+            # runs the problems segment by segment, not in their original
+            # order): the copies were queued on the side stream, wait for the
+            # last one
             torch.cuda.current_stream(x0.device).wait_event(plan[-1][2])
     else:
         options.pop("h2d_chunks", None)
@@ -274,12 +312,30 @@ def _least_squares_batched(lib, fun, x0, jac, bounds, method, ftol, xtol, gtol,
     if lb.shape != ub.shape:
         lb = lb.expand(B, n).contiguous()
         ub = ub.expand(B, n).contiguous()
-    if bool(torch.any(lb >= ub).item()):
+    cols = options.pop("cols", None)
+    used = None
+    if cols is not None:
+        # the coordinates past cols[b] are held fixed: their bounds and
+        # scaling are never read and not checked
+        cols = _check_cols(cols, B, n, x0.device)
+        used = torch.arange(n, device=x0.device)[None, :] < cols[:, None]
+    bad = lb >= ub
+    if used is not None:
+        bad = bad & (used if bad.dim() == 2 else used.any(0))
+    if bool(torch.any(bad).item()):
         raise ValueError("Each lower bound mush be strictly less than each "
                          "upper bound.")
-    scaling = check_scaling(scaling, x0)
+    scaling = check_scaling(scaling, x0,
+                            None if cols is None else int(cols.max().item()) if B else 0)
     ftol, xtol, gtol = check_tolerance(ftol, xtol, gtol)
-    if not bool(lib.in_bounds(x0, lb, ub).all().item()):
+    if used is None:
+        feasible = lib.in_bounds(x0, lb, ub)
+    else:
+        inf = torch.tensor(float("inf"), dtype=torch.float64, device=x0.device)
+        feasible = lib.in_bounds(torch.where(used, x0, 0.0).contiguous(),
+                                 torch.where(used, lb, -inf).contiguous(),
+                                 torch.where(used, ub, inf).contiguous())
+    if not bool(feasible.all().item()):
         raise ValueError("`x0` is infeasible.")
     for v in list(args) + list(dict(kwargs).values()):
         if isinstance(v, PerProblem):
@@ -291,7 +347,8 @@ def _least_squares_batched(lib, fun, x0, jac, bounds, method, ftol, xtol, gtol,
     cb = BatchedCallbacks(fun, jac, args, kwargs, B)
     jarg = jac if isinstance(jac, str) else cb.j
     out = solve_batched(lib, method, cb.f, jarg, x0, lb, ub, ftol, xtol, gtol,
-                        max_nfev, scaling, diff_step=diff_step, rows=rows, **options)
+                        max_nfev, scaling, diff_step=diff_step, rows=rows, cols=cols,
+                        **options)
     res = OptimizeResult(out)
     res.fun = cb.f(res.x, None)
     if rows is not None:
@@ -330,6 +387,26 @@ def _check_rows(rows, B, dev):
         if int(rows.max().item()) > 2 ** 31 - 1:
             raise ValueError("`rows` exceeds the number of residuals.")
     return rows.to(device=dev, dtype=torch.int32).contiguous()
+
+
+def _check_cols(cols, B, n, dev):
+    """``options['cols']``: an integer tensor of shape (B,) with every count
+    in 1 .. n, as a contiguous int32 tensor on ``dev``."""
+    if not isinstance(cols, torch.Tensor):
+        try:
+            cols = torch.as_tensor(cols)
+        except (TypeError, ValueError, RuntimeError):
+            raise ValueError("`cols` must be an integer tensor of shape (B,).")
+    if cols.dtype.is_floating_point or cols.dtype.is_complex or cols.dtype == torch.bool:
+        raise ValueError(f"`cols` must be an integer tensor, got {cols.dtype}.")
+    if tuple(cols.shape) != (B,):
+        raise ValueError(f"`cols` must have shape (B,) = ({B},), got {tuple(cols.shape)}.")
+    if B:
+        if int(cols.min().item()) < 1:
+            raise ValueError("`cols` must be at least 1 for every problem.")
+        if int(cols.max().item()) > n:
+            raise ValueError(f"`cols` exceeds the number of parameters n = {n}.")
+    return cols.to(device=dev, dtype=torch.int32).contiguous()
 
 
 _COPY_STREAM = {}

@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define BLSQ_VERSION 102
+#define BLSQ_VERSION 103
 
 #define BLSQ_E_BADARG (-1)      /* null pointer / negative size */
 #define BLSQ_E_UNSUPPORTED (-2) /* n outside 1..BLSQ_MAX_BATCHED_N, ... */
@@ -200,6 +200,60 @@ int blsq_round_batched_rows(int method, int64_t A, const int32_t* idx, int m, in
                             int first, double* state, int32_t* istate, double* Xnew,
                             double* Xjac, int32_t* work, int32_t* count,
                             const int32_t* rows, void* stream);
+
+/* Ragged parameter counts (version 103): a batch whose problems have their
+ * own number of parameters is solved as segments, one per count N, each a
+ * dense lock-step solve of N-parameter problems whose trial points share one
+ * padded (A, ldj) callback batch (least_squares_batched `cols`).
+ *
+ * blsq_linearise_batched_rows for the segment's slots of an (A, m, ldj)
+ * Jacobian: row r of slot s starts at J + (s * m + r) * ldj, and only its
+ * first n columns are read (the others may hold anything, NaN included).
+ * F, Fp_host, dx, lin, istate and rows are those of the n-parameter
+ * segment, as for blsq_linearise_batched_rows; the finite-difference modes
+ * do not read J, so ldj only matters for jac_mode 0.  With ldj == n (or
+ * jac_mode != 0) this is exactly blsq_linearise_batched_rows.  ldj < n is
+ * BLSQ_E_BADARG.  The record is bit for bit the one of a dense (A, m, n) J
+ * with the same columns.
+ * Alignment (jac_mode 0, ldj > n): a row start is only as aligned as ldj * 8
+ * bytes allows, so the rows are read with 4-double loads when 4 divides both
+ * n and ldj, 2-double loads when 2 does, else one double at a time; J must be
+ * aligned to that width (32 or 16 bytes), otherwise BLSQ_E_BADARG before any
+ * launch.  J aligned for the padded width ldj (blsq_linearise_batched) always
+ * is. */
+int blsq_linearise_batched_ld(int64_t A, const int32_t* idx, int m, int n, int ldj,
+                              const double* F, const double* J,
+                              const double* const* Fp_host, const double* dx,
+                              int jac_mode, const int32_t* istate, double* lin,
+                              const int32_t* rows, void* stream);
+
+/* One segment of a padded callback batch (blsq_pad_points): slots
+ * off .. off+A-1 of the batch hold its A active problems, in order. */
+typedef struct {
+    int64_t off;          /* first slot; segments tile 0 .. A-1 in order */
+    int64_t A;            /* its slots (0: an empty segment) */
+    int n;                /* its parameters, 1 <= n <= the padded width */
+    const int32_t* idx;   /* slot -> row of x0 (nullable: the slot itself) */
+    const double* x0;     /* its problems' x0, rows of the padded width */
+    const double* X;      /* (A, n) its points (Xnew / Xjac of its solve) */
+    const double* Xp;     /* (fd * n, A, n) its blsq_fd2_points / blsq_fd3_points
+                             batches; read only when fd != 0 */
+} blsq_pad_segment;
+
+/* The trial points of a ragged-parameter batch in the padded layout the
+ * callbacks take (no reference counterpart: the reference solves one problem
+ * of its own size per call).  nseg (1 .. BLSQ_MAX_BATCHED_N) segments from
+ * the HOST array seg_host; n is the padded width.  Coordinates k >= seg.n of
+ * every point are the problem's x0[k], unchanged (padded parameters are held
+ * fixed).
+ *   fd 0: out (A, n), slot s = X[s] padded.
+ *   fd 1: out (n, A, n), the 2-point batches: batch i of a segment with
+ *         seg.n > i is its Xp[i], of the others X (not perturbed: their
+ *         residuals at that batch are never read).
+ *   fd 2: out (2n, A, n), the 3-point batches 2i, 2i+1 likewise.
+ * The segments' offsets must tile 0 .. A-1; otherwise BLSQ_E_BADARG. */
+int blsq_pad_points(int nseg, const blsq_pad_segment* seg_host, int64_t A, int n, int fd,
+                    double* out, void* stream);
 
 /* dogbox.py:152-154,254: on_bound as the reference's int array (B x n) */
 int blsq_dogbox_on_bound(int64_t B, int n, const int32_t* istate,
