@@ -1,6 +1,7 @@
-// Batched mode kernels + C ABI (include/blsq.h) for sm_100a.
+// Batched mode C ABI (include/blsq.h) and its small kernels for sm_100a.
 //
-// Two kernels per round of the lock-step solve:
+// Two kernels per round of the lock-step solve, compiled once per parameter
+// count N in blsq_batched_n.cu:
 //
 //   lin_kernel    HBM-bound.  A group of 8/16/32 lanes owns one problem; the
 //                 lanes stream the rows of [J | f] with coalesced vector loads
@@ -232,36 +233,6 @@ __global__ void pad_points_kernel(PadTable tab, int64_t A, int n, int fd,
     }
 #endif
 
-namespace {
-
-// N = 9..16 are compiled in blsq_batched_wide.cu (one object per N)
-template <int N>
-int dispatch_lin(int64_t A, const int32_t* idx, int m, const double* F,
-                 const double* J, const double* const* Fp_host, const double* dx,
-                 int jac_mode, const int32_t* istate, double* lin,
-                 const int32_t* rows, cudaStream_t s) {
-    if constexpr (N <= 8)
-        return launch_lin<N>(A, idx, m, F, J, Fp_host, dx, jac_mode, istate, lin, rows, s);
-    else
-        return wide_launch_lin<N>(A, idx, m, F, J, Fp_host, dx, jac_mode, istate, lin, rows, s);
-}
-
-template <int N>
-int dispatch_round(int method, int64_t A, const int32_t* idx, const double* lin,
-                   const double* x0, const double* lb, const double* ub,
-                   int bstride, const double* scaling, SolveParams P, int first,
-                   double* state, int32_t* istate, double* Xnew, double* Xjac,
-                   int32_t* work, int32_t* count, const int32_t* rows, cudaStream_t s) {
-    if constexpr (N <= 8)
-        return launch_round<N>(method, A, idx, lin, x0, lb, ub, bstride, scaling, P, first,
-                               state, istate, Xnew, Xjac, work, count, rows, s);
-    else
-        return wide_launch_round<N>(method, A, idx, lin, x0, lb, ub, bstride, scaling, P,
-                                    first, state, istate, Xnew, Xjac, work, count, rows, s);
-}
-
-}  // namespace
-
 extern "C" {
 
 int blsq_state_layout(int method, int n, int* out) {
@@ -322,8 +293,8 @@ int blsq_linearise_batched_rows(int64_t A, const int32_t* idx, int m, int n,
             if (!Fp_host[j]) return BLSQ_E_BADARG;
     if (A == 0) return 0;
     BLSQ_DISPATCH_N(n, {
-        return dispatch_lin<N_>(A, idx, m, F, J, Fp_host, dx, jac_mode, istate,
-                                lin, rows, (cudaStream_t)stream);
+        return batched_lin<N_>(A, idx, m, n, F, J, Fp_host, dx, jac_mode, istate,
+                               lin, rows, (cudaStream_t)stream);
     });
     return 0;
 }
@@ -351,14 +322,11 @@ int blsq_linearise_batched_ld(int64_t A, const int32_t* idx, int m, int n, int l
     // width follows from both n and ldj, and J must be aligned to it
     if ((uintptr_t)J % (8 * lin_ld_width(n, ldj))) return BLSQ_E_BADARG;
     if (A == 0) return 0;
-#ifdef BLSQ_ONLY_N46
-    return BLSQ_E_UNSUPPORTED;
-#else
     BLSQ_DISPATCH_N(n, {
-        return ld_launch_lin<N_>(A, idx, m, ldj, F, J, istate, lin, rows, (cudaStream_t)stream);
+        return batched_lin<N_>(A, idx, m, ldj, F, J, Fp_host, dx, jac_mode, istate, lin,
+                               rows, (cudaStream_t)stream);
     });
     return 0;
-#endif
 }
 
 int blsq_pad_points(int nseg, const blsq_pad_segment* seg_host, int64_t A, int n, int fd,
@@ -405,9 +373,9 @@ int blsq_round_batched_rows(int method, int64_t A, const int32_t* idx, int m, in
     P.ftol = ftol; P.xtol = xtol; P.gtol = gtol;
     P.max_nfev = max_nfev; P.m = m; P.jac_scaling = scaling ? 0 : 1;
     BLSQ_DISPATCH_N(n, {
-        return dispatch_round<N_>(method, A, idx, lin, x0, lb, ub, bstride,
-                                  scaling, P, first, state, istate, Xnew, Xjac,
-                                  work, count, rows, (cudaStream_t)stream);
+        return batched_round<N_>(method, A, idx, lin, x0, lb, ub, bstride,
+                                 scaling, P, first, state, istate, Xnew, Xjac,
+                                 work, count, rows, (cudaStream_t)stream);
     });
     return 0;
 }
@@ -471,16 +439,3 @@ int blsq_compact_batched(int64_t A, const int32_t* idx, const int32_t* istate, i
 }
 
 }  // extern "C"
-
-#ifdef BLSQ_PHASE_CLOCKS
-// tools/phase_probe.py only: cycles [0..15] and visits [16..31] per phase of
-// trf_round_impl since the last reset
-extern "C" int blsq_debug_phase_read(unsigned long long* out, int reset) {
-    cudaError_t e = cudaMemcpyFromSymbol(out, blsq_phase_acc, sizeof(blsq_phase_acc));
-    if (e == cudaSuccess && reset) {
-        unsigned long long z[32] = {0};
-        e = cudaMemcpyToSymbol(blsq_phase_acc, z, sizeof(z));
-    }
-    return (int)e;
-}
-#endif

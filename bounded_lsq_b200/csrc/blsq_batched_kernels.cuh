@@ -1,7 +1,7 @@
 // Batched mode: the templated round kernel and the launchers of lin_kernel and
-// round_kernel, shared by blsq_batched.cu (N = 1..8, and the C ABI) and
-// blsq_batched_wide.cu (N = 9..16, one object per N so that make -j compiles
-// them in parallel).
+// round_kernel, instantiated by blsq_batched_n.cu once per N (one object per N,
+// so that make -j compiles them in parallel), and the two entry points of each
+// N that the C ABI in blsq_batched.cu calls.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -226,14 +226,15 @@ round_kernel(int64_t A, const int32_t* __restrict__ idx,
     }
 }
 
-template <int N, int G, bool MULTI, bool ROWS>
-int launch_lin_r(unsigned blocks, int64_t A, const int32_t* idx, int m, const double* F,
-                 const double* J, const PtrList<N>& pl, const double* dx,
+// LDW > 0: J padded to ldj > N columns (MODE 0 only)
+template <int N, int G, bool MULTI, bool ROWS, int LDW = 0>
+int launch_lin_r(unsigned blocks, int64_t A, const int32_t* idx, int m, int ldj,
+                 const double* F, const double* J, const PtrList<N>& pl, const double* dx,
                  int jac_mode, const int32_t* istate, double* lin,
                  const int32_t* rows, cudaStream_t s) {
-    if (jac_mode == 0)
-        lin_kernel<N, G, 0, MULTI, NoModel, ROWS><<<blocks, BLSQ_LIN_THREADS, 0, s>>>(
-            A, idx, m, F, J, pl, dx, istate, lin, NoModel(), rows);
+    if (LDW || jac_mode == 0)
+        lin_kernel<N, G, 0, MULTI, NoModel, ROWS, LDW><<<blocks, BLSQ_LIN_THREADS, 0, s>>>(
+            A, idx, m, F, J, pl, dx, istate, lin, NoModel(), rows, ldj);
     else if (jac_mode == 1)
         lin_kernel<N, G, 1, MULTI, NoModel, ROWS><<<blocks, BLSQ_LIN_THREADS, 0, s>>>(
             A, idx, m, F, J, pl, dx, istate, lin, NoModel(), rows);
@@ -244,44 +245,38 @@ int launch_lin_r(unsigned blocks, int64_t A, const int32_t* idx, int m, const do
     return 0;
 }
 
-// rows == null: the dense instances; else the ragged ones (lin_kernel ROWS)
+// MODE 0 with ldj != N: the LD instance of width lin_ld_width(N, ldj) (rows
+// may be null there); else rows == null: the dense instances, and otherwise
+// the ragged ones (lin_kernel ROWS)
 template <int N, int G, bool MULTI>
-int launch_lin_g(int64_t A, const int32_t* idx, int m, const double* F,
+int launch_lin_g(int64_t A, const int32_t* idx, int m, int ldj, const double* F,
                  const double* J, const PtrList<N>& pl, const double* dx,
                  int jac_mode, const int32_t* istate, double* lin,
                  const int32_t* rows, cudaStream_t s) {
     int64_t threads = A * G;
     int64_t blocks = (threads + BLSQ_LIN_THREADS - 1) / BLSQ_LIN_THREADS;
     if (blocks > 0x7fffffff) return BLSQ_E_UNSUPPORTED;
-    if (rows)
-        return launch_lin_r<N, G, MULTI, true>((unsigned)blocks, A, idx, m, F, J, pl, dx,
-                                               jac_mode, istate, lin, rows, s);
-    return launch_lin_r<N, G, MULTI, false>((unsigned)blocks, A, idx, m, F, J, pl, dx,
-                                            jac_mode, istate, lin, nullptr, s);
-}
-
-template <int N>
-int launch_lin(int64_t A, const int32_t* idx, int m, const double* F,
-               const double* J, const double* const* Fp_host, const double* dx,
-               int jac_mode, const int32_t* istate, double* lin,
-               const int32_t* rows, cudaStream_t s) {
-    constexpr int RPL = LinCfg<N>::RPL;
-    PtrList<N> pl;
-    const int np = jac_mode == 2 ? 2 * N : (jac_mode == 1 ? N : 0);
-    for (int j = 0; j < 2 * N; j++) pl.p[j] = (j < np) ? Fp_host[j] : nullptr;
-    // smallest lane group whose registers hold all m rows (else 32 + chunks);
-    // a ragged batch is classed by its width m, not by its counts.  N > 8
-    // has no 8-lane class: lane k stores row k of R (lin_kernel)
-    if constexpr (N <= 8) {
-        if (m <= 8 * RPL)
-            return launch_lin_g<N, 8, false>(A, idx, m, F, J, pl, dx, jac_mode, istate, lin,
-                                             rows, s);
+    const unsigned b = (unsigned)blocks;
+    if (jac_mode == 0 && ldj != N) {
+        const int w = lin_ld_width(N, ldj);
+        if constexpr (N % 4 == 0) {
+            if (w == 4)
+                return launch_lin_r<N, G, MULTI, true, 4>(b, A, idx, m, ldj, F, J, pl, dx,
+                                                          jac_mode, istate, lin, rows, s);
+        }
+        if constexpr (N % 2 == 0) {
+            if (w == 2)
+                return launch_lin_r<N, G, MULTI, true, 2>(b, A, idx, m, ldj, F, J, pl, dx,
+                                                          jac_mode, istate, lin, rows, s);
+        }
+        return launch_lin_r<N, G, MULTI, true, 1>(b, A, idx, m, ldj, F, J, pl, dx, jac_mode,
+                                                  istate, lin, rows, s);
     }
-    if (m <= 16 * RPL)
-        return launch_lin_g<N, 16, false>(A, idx, m, F, J, pl, dx, jac_mode, istate, lin, rows, s);
-    if (m <= 32 * RPL)
-        return launch_lin_g<N, 32, false>(A, idx, m, F, J, pl, dx, jac_mode, istate, lin, rows, s);
-    return launch_lin_g<N, 32, true>(A, idx, m, F, J, pl, dx, jac_mode, istate, lin, rows, s);
+    if (rows)
+        return launch_lin_r<N, G, MULTI, true>(b, A, idx, m, ldj, F, J, pl, dx, jac_mode,
+                                               istate, lin, rows, s);
+    return launch_lin_r<N, G, MULTI, false>(b, A, idx, m, ldj, F, J, pl, dx, jac_mode,
+                                            istate, lin, nullptr, s);
 }
 
 template <int N, bool ROWS>
@@ -319,38 +314,19 @@ int launch_round_r(int method, int64_t A, const int32_t* idx, const double* lin,
     return 0;
 }
 
-// rows == null: the dense instances; else the ragged ones (round_slot ROWS)
-template <int N>
-int launch_round(int method, int64_t A, const int32_t* idx, const double* lin,
-                 const double* x0, const double* lb, const double* ub,
-                 int bstride, const double* scaling, SolveParams P, int first,
-                 double* state, int32_t* istate, double* Xnew, double* Xjac,
-                 int32_t* work, int32_t* count, const int32_t* rows, cudaStream_t s) {
-    if (rows)
-        return launch_round_r<N, true>(method, A, idx, lin, x0, lb, ub, bstride, scaling, P,
-                                       first, state, istate, Xnew, Xjac, work, count, rows, s);
-    return launch_round_r<N, false>(method, A, idx, lin, x0, lb, ub, bstride, scaling, P,
-                                    first, state, istate, Xnew, Xjac, work, count, nullptr, s);
-}
-
 }  // namespace
 
-// lin_kernel for a Jacobian padded to ldj > N columns (blsq_linearise_batched_ld),
-// defined in blsq_batched_ld.cu, one object per N
+// The lin_kernel and round_kernel instances of parameter count N, one object
+// per N (blsq_batched_n.cu).  batched_lin: ldj is the row stride of J (N for
+// a dense Jacobian; > N, MODE 0 only, for one padded to more columns).
 template <int N>
-int ld_launch_lin(int64_t A, const int32_t* idx, int m, int ldj, const double* F,
-                  const double* J, const int32_t* istate, double* lin,
-                  const int32_t* rows, cudaStream_t s);
-
-// the instances for N = 9..16, defined in blsq_batched_wide.cu
+int batched_lin(int64_t A, const int32_t* idx, int m, int ldj, const double* F,
+                const double* J, const double* const* Fp_host, const double* dx,
+                int jac_mode, const int32_t* istate, double* lin,
+                const int32_t* rows, cudaStream_t s);
 template <int N>
-int wide_launch_lin(int64_t A, const int32_t* idx, int m, const double* F,
-                    const double* J, const double* const* Fp_host, const double* dx,
-                    int jac_mode, const int32_t* istate, double* lin,
-                    const int32_t* rows, cudaStream_t s);
-template <int N>
-int wide_launch_round(int method, int64_t A, const int32_t* idx, const double* lin,
-                      const double* x0, const double* lb, const double* ub,
-                      int bstride, const double* scaling, SolveParams P, int first,
-                      double* state, int32_t* istate, double* Xnew, double* Xjac,
-                      int32_t* work, int32_t* count, const int32_t* rows, cudaStream_t s);
+int batched_round(int method, int64_t A, const int32_t* idx, const double* lin,
+                  const double* x0, const double* lb, const double* ub,
+                  int bstride, const double* scaling, SolveParams P, int first,
+                  double* state, int32_t* istate, double* Xnew, double* Xjac,
+                  int32_t* work, int32_t* count, const int32_t* rows, cudaStream_t s);

@@ -1,8 +1,8 @@
 // Batched mode, the linearisation kernel (HBM bound): QR of [J | f] per
 // problem with the rows in registers.  A header so that a residual model can be
 // compiled INTO the kernel (MODE 3, blsq_models.cu: J never touches HBM); the
-// library's own entry point blsq_linearise_batched (blsq_batched.cu) uses
-// modes 0 - 2 with NoModel.
+// library's own instances (blsq_batched_n.cu, one object per N) use modes
+// 0 - 2 with NoModel.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -45,8 +45,8 @@ template <int N, bool WIDE = (N > 8)> struct LinCfg {
     static constexpr int RPL = (N <= 4) ? BLSQ_RPL_SMALL : (N <= 6 ? BLSQ_RPL_MID : 4);
     static constexpr int MINB = (N <= 4 || RPL <= 4) ? BLSQ_LIN_MINB : BLSQ_LIN_MINB_MID;
 };
-// N = 9..16 (blsq_batched_wide.cu; lane groups of 16 / 32 only): 4 rows per
-// lane up to N = 12, then 2, at 2 CTAs / SM (255 registers).  The largest
+// N = 9..16 (lane groups of 16 / 32 only): 4 rows per lane up to N = 12,
+// then 2, at 2 CTAs / SM (255 registers).  The largest
 // budgets without spills in any of the 18 instances of an N: 4 rows at 3 CTAs
 // spill 1.3-1.5 KB at N = 12 in MULTI, 4 rows spill at N = 16 even at 2 CTAs
 // (profiles/r4_wide_ptxas.md).

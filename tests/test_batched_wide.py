@@ -1,6 +1,6 @@
 """Batched mode for 9 <= n <= 16 parameters per problem.
 
-The instances for N = 9..16 (csrc/blsq_batched_wide.cu) have their own
+The lin_kernel instances for N = 9..16 (csrc/blsq_batched_n.cu) have their own
 lin_kernel class table: lane groups of 16 or 32 and MULTI, no 8-lane class
 (lane k stores row k of R), with LinCfg<N, true>::RPL rows per lane.  The
 round kernel runs the per-thread code of N <= 8.
@@ -48,7 +48,7 @@ def rpl(N):
 
 
 def lin_class(N, m):
-    """The class launch_lin picks for N > 8: the smallest group of 16 or 32
+    """The class batched_lin picks for N > 8: the smallest group of 16 or 32
     lanes whose registers hold all m rows, else MULTI."""
     for G, name in ((16, "G16"), (32, "G32")):
         if m <= G * rpl(N):

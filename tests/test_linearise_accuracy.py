@@ -2,7 +2,7 @@
 
 lin_kernel (csrc/blsq_lin.cuh) turns [J | f] of every running problem into the
 record the round kernel works from (LinRec<N>): R packed row-major from 0, Q^T f
-at NT, g = J^T f at NT + N and f.f at NT + 2N.  launch_lin picks one of
+at NT, g = J^T f at NT + N and f.f at NT + 2N.  batched_lin picks one of
 8 N x 4 lane-group classes x 3 Jacobian modes x {dense, ROWS} instances; the
 checks below call blsq_linearise_batched[_rows] directly at both sides of every
 class edge for every N.
@@ -42,7 +42,7 @@ def rpl(N):
 
 
 def lin_class(N, m):
-    """The lane-group class launch_lin picks: the smallest group whose
+    """The lane-group class batched_lin picks: the smallest group whose
     registers hold all m rows, else 32 lanes folding chunks (MULTI)."""
     for G, name in ((8, "G8"), (16, "G16"), (32, "G32")):
         if m <= G * rpl(N):
