@@ -82,16 +82,25 @@ class BatchedCallbacks:
         a, k = self._gathered[1]
         return fn(X, *a, **k)
 
-    def lin(self, X, idx32, off, A, p_istate, p_lin, stream):
+    def lin(self, X, Xjac, Xp, dx, idx32, off, A, p_istate, p_lin, stream):
         """Models compiled into the linearisation kernel (``fun.blsq_linearise``,
         bounded_lsq_b200.models): returns m when the callbacks of this round
-        and blsq_linearise_batched were replaced by that one launch, else None."""
+        and blsq_linearise_batched were replaced by that one launch, else None.
+
+        The hook is called as ``fn(X, Xjac, Xp, dx, idx32, p_istate, p_lin,
+        stream, *args, **kwargs)`` with the raw per-problem data: f at the
+        (A, n) trial points X; J analytic at Xjac (dogbox's bound-snapped
+        points; None for TRF: at X), or, with Xp and dx given, by 2-point
+        differences from the (n, A, n) points and (A, n) steps of
+        blsq_fd2_points.  It writes the records of the running problems among
+        the A slots (idx32: slot -> problem id, None for the identity) and
+        returns m, or returns None to decline the round."""
         fn = getattr(self.fun, "blsq_linearise", None)
         if fn is None:
             return None
         sl = slice(off, off + A) if (idx32 is None and (off or A != self.B)) else slice(None)
         a, k = self._raw_args(sl)
-        return fn(X, idx32, p_istate, p_lin, stream, *a, **k)
+        return fn(X, Xjac, Xp, dx, idx32, p_istate, p_lin, stream, *a, **k)
 
     def f(self, X, idx):
         return self._call(self.fun, X, idx)
@@ -394,14 +403,35 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
                 rows=None if g.rows is None else g.rows.data_ptr() + off * 4,
                 ip=None if g.idx32 is None else g.idx32.data_ptr())
         P = [ptrs(g) for g, _ in live]
-        # a model compiled into the linearisation kernel replaces the two
-        # callbacks and blsq_linearise_batched of this round by one launch
+        def fd_points():
+            """blsq_fd2_points / blsq_fd3_points: every segment's perturbed
+            points (g.Xp) and steps (g.dx) at the points J is evaluated at."""
+            nonlocal launches
+            for (g, a), p in zip(live, P):
+                Xpa = g.Xp.view(-1)[: g.npts * a * g.N].view(g.npts, a, g.N)
+                lib.call("blsq_fd3_points" if fd3 else "blsq_fd2_points", a, p["ip"],
+                         g.N, (xj(g) if padded else Xj).data_ptr(),
+                         p["lb"], p["ub"], g.bs, rel, Xpa.data_ptr(), g.dx.data_ptr(),
+                         stream)
+                launches += 1
+            return Xpa
+
+        # a model compiled into the linearisation kernel replaces the
+        # callbacks and blsq_linearise_batched of this round by one launch;
+        # with 2-point differences it is offered the points before fun runs
         cbs = getattr(fun, "__self__", None)
+        hook = not padded and segs[0].rows is None and \
+            getattr(getattr(cbs, "fun", None), "blsq_linearise", None) is not None
         mm = None
-        if not padded and not fd and segs[0].Xjac is None and segs[0].rows is None \
-                and hasattr(cbs, "lin"):
+        Xpa = None
+        if hook and (not fd or not fd3):
+            g = segs[0]
+            if fd:
+                Xpa = fd_points()
             t0 = tick()
-            mm = cbs.lin(Xa, segs[0].idx32, off, A, P[0]["ist"], P[0]["lin"], stream)
+            mm = cbs.lin(Xa, None if (fd or g.Xjac is None) else Xj, Xpa,
+                         g.dx if fd else None, g.idx32, off, A, P[0]["ist"], P[0]["lin"],
+                         stream)
             if mm is not None:
                 m = mm
                 launches += 1
@@ -442,13 +472,8 @@ def solve_batched(lib, method, fun, jac, X0, lb, ub, ftol, xtol, gtol,
                     tock("linearise", t0, nrun, g if padded else None)
                     s0 += a
             else:
-                for (g, a), p in zip(live, P):
-                    Xpa = g.Xp.view(-1)[: g.npts * a * g.N].view(g.npts, a, g.N)
-                    lib.call("blsq_fd3_points" if fd3 else "blsq_fd2_points", a, p["ip"],
-                             g.N, (xj(g) if padded else Xj).data_ptr(),
-                             p["lb"], p["ub"], g.bs, rel, Xpa.data_ptr(), g.dx.data_ptr(),
-                             stream)
-                    launches += 1
+                if Xpa is None:                # not yet written for a hook
+                    Xpa = fd_points()
                 npts = 2 * n if fd3 else n
                 if padded:
                     Xpa = Xpcb.view(-1)[: npts * A * n].view(npts, A, n)

@@ -19,26 +19,14 @@ int batched_lin(int64_t A, const int32_t* idx, int m, int ldj, const double* F,
                 const double* J, const double* const* Fp_host, const double* dx,
                 int jac_mode, const int32_t* istate, double* lin,
                 const int32_t* rows, cudaStream_t s) {
-    constexpr int RPL = LinCfg<N>::RPL;
     PtrList<N> pl;
     const int np = jac_mode == 2 ? 2 * N : (jac_mode == 1 ? N : 0);
     for (int j = 0; j < 2 * N; j++) pl.p[j] = (j < np) ? Fp_host[j] : nullptr;
-    // smallest lane group whose registers hold all m rows (else 32 + chunks);
-    // a ragged batch is classed by its width m, not by its counts.  N > 8
-    // has no 8-lane class: lane k stores row k of R (lin_kernel)
-    if constexpr (N <= 8) {
-        if (m <= 8 * RPL)
-            return launch_lin_g<N, 8, false>(A, idx, m, ldj, F, J, pl, dx, jac_mode, istate,
-                                             lin, rows, s);
-    }
-    if (m <= 16 * RPL)
-        return launch_lin_g<N, 16, false>(A, idx, m, ldj, F, J, pl, dx, jac_mode, istate, lin,
-                                          rows, s);
-    if (m <= 32 * RPL)
-        return launch_lin_g<N, 32, false>(A, idx, m, ldj, F, J, pl, dx, jac_mode, istate, lin,
-                                          rows, s);
-    return launch_lin_g<N, 32, true>(A, idx, m, ldj, F, J, pl, dx, jac_mode, istate, lin,
-                                     rows, s);
+    // a ragged batch is classed by its width m, not by its counts
+    return lin_class<N>(m, [&](auto g, auto multi) {
+        return launch_lin_g<N, decltype(g)::value, decltype(multi)::value>(
+            A, idx, m, ldj, F, J, pl, dx, jac_mode, istate, lin, rows, s);
+    });
 }
 
 // rows == null: the dense instances; else the ragged ones (round_slot ROWS)

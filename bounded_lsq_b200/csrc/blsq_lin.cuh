@@ -7,6 +7,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <type_traits>
+
 #include "blsq_core.cuh"
 
 namespace blsq_lin {
@@ -96,6 +98,24 @@ __device__ __forceinline__ double div_rn(double a, double b, double y) {
     q = fma(fma(-b, q, a), y, q);
     q = fma(fma(-b, q, a), y, q);
     return q;
+}
+
+// The lane-group class of lin_kernel for m rows: the smallest group whose
+// registers hold all m rows, else 32 lanes that fold the rows in chunk by
+// chunk (MULTI).  N > 8 has no 8-lane class: lane k stores row k of R.
+// Returns launch(std::integral_constant<int, G>(), std::bool_constant<MULTI>()).
+// The one place the class is chosen: the library's instances
+// (batched_lin) and compiled user models (blsq_user_model.cuh) both use it.
+template <int N, class Launch>
+int lin_class(int m, Launch&& launch) {
+    constexpr int RPL = LinCfg<N>::RPL;
+    if constexpr (N <= 8) {
+        if (m <= 8 * RPL)
+            return launch(std::integral_constant<int, 8>(), std::false_type());
+    }
+    if (m <= 16 * RPL) return launch(std::integral_constant<int, 16>(), std::false_type());
+    if (m <= 32 * RPL) return launch(std::integral_constant<int, 32>(), std::false_type());
+    return launch(std::integral_constant<int, 32>(), std::true_type());
 }
 
 template <int N> struct PtrList { const double* p[2 * N]; };   // 2 per coordinate (3-point)

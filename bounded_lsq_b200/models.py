@@ -1,5 +1,10 @@
 """Fused CUDA residual/Jacobian callbacks for the synthetic workloads.
 
+``compile_model`` compiles a residual model written by the user as a small
+CUDA C++ struct (contract: ``csrc/blsq_user_model.cuh``) into callbacks of the
+same protocol, whose inlined kinds run the model inside the linearisation
+kernel.
+
 User-side code (include/blsq_models.h): the same functions as
 ``synthetic.ExpDecay2.fun_t/jac_t`` and ``synthetic.GaussPeak.fun_t`` as one
 kernel each, with the active-set gather of the per-problem data fused into
@@ -8,6 +13,13 @@ the load.  They use the *indexed* callback protocol of the batched driver:
 per-problem tensors plus the active problem ids instead of gathered copies.
 """
 from __future__ import annotations
+
+import ctypes as C
+import hashlib
+import os
+import shutil
+import subprocess
+import tempfile
 
 import torch
 
@@ -98,10 +110,14 @@ def callbacks(model_name, jac_kind="exact", lib=None, rows=False):
         if not lib.has("blsq_model_expdecay2_linearise"):
             raise L.BlsqError("library built without the inlined ExpDecay2 linearisation")
 
-        def linearise(X, idx32, p_istate, p_lin, stream, y):
+        def linearise(X, Xjac, Xp, dx, idx32, p_istate, p_lin, stream, y):
             """The lin records of the trial points X straight from (X, t, y): the
             model is compiled into the linearisation kernel, J and f never
-            touch HBM.  Same bits as fun + jac + blsq_linearise_batched."""
+            touch HBM.  Same bits as fun + jac + blsq_linearise_batched.  TRF
+            rounds only: dogbox's Jacobian points and finite differences are
+            declined (None), those rounds call fun and jac."""
+            if Xjac is not None or Xp is not None:
+                return None
             t = _t_on(model, X.device, tcache)
             lib.call("blsq_model_expdecay2_linearise", X.shape[0],
                      None if idx32 is None else idx32.data_ptr(), model.m,
@@ -142,3 +158,212 @@ def tall_callbacks(wl, lib=None):
         return wl.J_t
 
     return fun, jac
+
+
+# ---- residual models compiled from user source ------------------------------
+
+_PKG = os.path.dirname(os.path.abspath(__file__))
+_CSRC = os.path.join(_PKG, "csrc")
+# what a compiled model is built from besides its source: part of the cache key
+_HEADERS = [os.path.join(_CSRC, f) for f in ("blsq_user_model.cuh", "blsq_lin.cuh",
+                                             "blsq_core.cuh", "Makefile")] + \
+           [os.path.join(_PKG, "..", "include", "blsq.h")]
+MAX_DATA = 8                              # BLSQ_MODEL_MAX_DATA
+KINDS = ("exact", "2-point", "3-point", "inlined", "inlined-2-point")
+_NVCC_VERSION = {}
+_LOADED = {}
+
+
+def _nvcc():
+    """The nvcc that `make` in csrc/ runs for the library: $NVCC, else PATH."""
+    exe = shutil.which(os.environ.get("NVCC", "nvcc"))
+    if exe is None:
+        raise L.BlsqError("nvcc not found: compile_model needs the CUDA toolkit "
+                          "that builds the library (nvcc on PATH or $NVCC)")
+    if exe not in _NVCC_VERSION:
+        _NVCC_VERSION[exe] = subprocess.run([exe, "--version"], capture_output=True,
+                                            text=True, check=True).stdout
+    return exe, _NVCC_VERSION[exe]
+
+
+def _default_cache_dir():
+    base = os.environ.get("XDG_CACHE_HOME") or os.path.join(os.path.expanduser("~"), ".cache")
+    return os.path.join(base, "bounded_lsq_b200", "models")
+
+
+def generated_source(source, name="Model"):
+    """The .cu that compile_model builds: the contract header, the user's
+    source (diagnostics point at its own lines) and the entry points."""
+    if not name.isidentifier():
+        raise ValueError(f"model name {name!r} is not a C++ identifier")
+    return ('#include "blsq_user_model.cuh"\n'
+            '#line 1 "model.cu"\n'
+            f"{source}\n"
+            f"BLSQ_USER_MODEL_ENTRY_POINTS({name})\n")
+
+
+def compile_model(source, name="Model", cache_dir=None):
+    """Compile the residual model ``name`` defined in ``source`` (CUDA C++,
+    contract in ``csrc/blsq_user_model.cuh``) for sm_100a with the library's
+    own flags and return a :class:`CompiledModel`.
+
+    The shared object is cached under ``cache_dir`` (default: a per-user cache
+    directory) by a hash of the generated source, the headers it includes, the
+    Makefile (the flags) and ``nvcc --version``; a cached object is loaded
+    without running nvcc.  It is written under a temporary name and renamed,
+    so concurrent processes compiling the same model do not collide.  A
+    compile error raises BlsqError with nvcc's diagnostics."""
+    cu = generated_source(source, name)
+    nvcc, version = _nvcc()
+    h = hashlib.sha256()
+    for part in [cu.encode(), version.encode()] + [open(p, "rb").read() for p in _HEADERS]:
+        h.update(hashlib.sha256(part).digest())
+    key = h.hexdigest()[:32]
+    cache_dir = os.path.abspath(cache_dir or _default_cache_dir())
+    path = os.path.join(cache_dir, f"blsq_model_{key}.so")
+    log = path[:-3] + ".ptxas.log"
+    built = False
+    if not os.path.exists(path):
+        os.makedirs(cache_dir, exist_ok=True)
+        with tempfile.TemporaryDirectory(dir=cache_dir, prefix=".build-") as tmp:
+            src = os.path.join(tmp, "model.cu")
+            with open(src, "w") as f:
+                f.write(cu)
+            out = os.path.join(tmp, "model.so")
+            r = subprocess.run(["make", "-s", "-C", _CSRC, "user-model", f"NVCC={nvcc}",
+                                f"SRC={src}", f"OUT={out}"], capture_output=True, text=True)
+            if r.returncode != 0 or not os.path.exists(out):
+                raise L.BlsqError(f"compile_model({name!r}): nvcc failed\n{r.stderr}{r.stdout}")
+            with open(os.path.join(tmp, "ptxas.log"), "w") as f:
+                f.write(r.stderr)
+            os.replace(os.path.join(tmp, "ptxas.log"), log)
+            os.replace(out, path)
+        built = True
+    if path not in _LOADED:
+        _LOADED[path] = C.CDLL(path)
+    return CompiledModel(_LOADED[path], path, name, built)
+
+
+_p, _i, _l = C.c_void_p, C.c_int, C.c_int64
+_UM_SIGNATURES = {
+    "blsq_um_info": [_p],
+    "blsq_um_linearise": [_l, _p, _i, _p, _p, _p, _i, _p, _p, _p],
+    "blsq_um_linearise_fd2": [_l, _p, _i, _p, _p, _p, _p, _i, _p, _p, _p],
+    "blsq_um_fun": [_l, _p, _i, _p, _p, _i, _p, _p],
+    "blsq_um_jac": [_l, _p, _i, _p, _p, _i, _p, _p],
+}
+
+
+class CompiledModel:
+    """A residual model compiled by :func:`compile_model`.
+
+    ``n``: its number of parameters; ``has_jacobian``: whether it defines
+    ``jacobian_row``; ``path``: the shared object; ``built``: whether this
+    call ran nvcc (False: loaded from the cache)."""
+
+    def __init__(self, dll, path, name, built):
+        self._dll, self.path, self.name, self.built = dll, path, name, built
+        for fn, args in _UM_SIGNATURES.items():
+            getattr(dll, fn).argtypes = args
+            getattr(dll, fn).restype = _i
+        dll.blsq_um_error_string.argtypes = [_i]
+        dll.blsq_um_error_string.restype = C.c_char_p
+        info = (C.c_int * 3)()
+        dll.blsq_um_info(info)
+        self.n, self.has_jacobian, self.version = info[0], bool(info[1]), info[2]
+
+    def _call(self, fn, *args):
+        rc = getattr(self._dll, fn)(*args)
+        if rc != 0:
+            msg = self._dll.blsq_um_error_string(rc).decode()
+            raise L.BlsqError(f"{self.name}: {fn} failed: {msg} (code {rc})")
+
+    def _data(self, X, data):
+        if len(data) > MAX_DATA:
+            raise ValueError(f"a compiled model takes at most {MAX_DATA} data tensors, "
+                             f"got {len(data)}")
+        for k, d in enumerate(data):
+            if not isinstance(d, torch.Tensor) or d.dtype != torch.float64 \
+                    or not d.is_contiguous() or not d.is_cuda or d.device != X.device:
+                raise ValueError(
+                    f"data argument {k} of a compiled model must be a contiguous float64 "
+                    f"tensor on the solve's CUDA device {X.device} (a PerProblem or shared "
+                    "argument), got "
+                    + (f"{d.dtype} on {d.device}" if isinstance(d, torch.Tensor)
+                       else type(d).__name__))
+        return (C.c_void_p * MAX_DATA)(*[d.data_ptr() for d in data]), len(data)
+
+    def callbacks(self, jac_kind, m, lib=None):
+        """(fun, jac) for ``least_squares_batched(fun, x0, jac=jac, args=data)``
+        with m residuals per problem, as ``models.callbacks`` returns them:
+
+        * ``'exact'``: materialised F and J kernels (needs ``jacobian_row``);
+        * ``'2-point'``, ``'3-point'``: the materialised F kernel and the
+          scheme's name; the solver forms the differences;
+        * ``'inlined'``: the model compiled into the linearisation kernel,
+          J and f never reach HBM (needs ``jacobian_row``);
+        * ``'inlined-2-point'``: 2-point differences formed in registers in
+          the linearisation kernel, f and the perturbed batches never reach HBM.
+
+        The data (the callbacks' ``args``: at most 8 contiguous float64 tensors
+        on the solve's device, ``PerProblem`` or shared) reach the model as
+        ``blsq_model_ctx::data`` in order.  The inlined kinds serve every
+        round of a dense TRF or dogbox solve; they do not take ``rows`` or
+        ``cols``."""
+        if jac_kind not in KINDS:
+            raise ValueError(f"jac_kind must be one of {KINDS}, got {jac_kind!r}")
+        if jac_kind in ("exact", "inlined") and not self.has_jacobian:
+            raise ValueError(f"{self.name} defines no jacobian_row: jac_kind "
+                             f"{jac_kind!r} needs one (use '2-point' or 'inlined-2-point')")
+        m = int(m)
+        if m < 1:
+            raise ValueError("m must be >= 1")
+        lib = lib or L.get_lib()
+        if not lib.requires_cuda:
+            raise L.BlsqError("compiled models run on CUDA devices only; the "
+                              "host-emulation library cannot run them")
+        n = self.n
+
+        def run(entry, X, idx, data, shape):
+            ptrs, nd = self._data(X, data)
+            X = X.contiguous()
+            out = torch.empty(shape, dtype=torch.float64, device=X.device)
+            self._call(entry, X.shape[0], None if idx is None else idx.data_ptr(), m,
+                       X.data_ptr(), ptrs, nd, out.data_ptr(), lib.stream(X))
+            return out
+
+        def fun(X, idx, *data):
+            return run("blsq_um_fun", X, idx, data, (X.shape[0], m))
+
+        def jac(X, idx, *data):
+            return run("blsq_um_jac", X, idx, data, (X.shape[0], m, n))
+
+        fun.blsq_indexed = True
+        jac.blsq_indexed = True
+        if jac_kind == "inlined":
+            def linearise(X, Xjac, Xp, dx, idx32, p_istate, p_lin, stream, *data):
+                """lin records of the trial points X, J at Xjac (dogbox) or X."""
+                if Xp is not None:
+                    return None
+                ptrs, nd = self._data(X, data)
+                self._call("blsq_um_linearise", X.shape[0],
+                           None if idx32 is None else idx32.data_ptr(), m, X.data_ptr(),
+                           None if Xjac is None else Xjac.data_ptr(), ptrs, nd,
+                           p_istate, p_lin, stream)
+                return m
+            fun.blsq_linearise = linearise
+        elif jac_kind == "inlined-2-point":
+            def linearise(X, Xjac, Xp, dx, idx32, p_istate, p_lin, stream, *data):
+                """lin records from f at X and at the 2-point batches Xp."""
+                if Xp is None:
+                    return None
+                ptrs, nd = self._data(X, data)
+                self._call("blsq_um_linearise_fd2", X.shape[0],
+                           None if idx32 is None else idx32.data_ptr(), m, X.data_ptr(),
+                           Xp.data_ptr(), dx.data_ptr(), ptrs, nd, p_istate, p_lin, stream)
+                return m
+            fun.blsq_linearise = linearise
+            return fun, "2-point"
+        if jac_kind in ("2-point", "3-point"):
+            return fun, jac_kind
+        return fun, jac
