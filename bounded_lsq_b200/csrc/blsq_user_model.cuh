@@ -14,6 +14,17 @@
 //                                    const blsq_model_ctx& c, double (&j)[N]) const;
 //   };
 //
+// The residual may instead be a template on its scalar type,
+//
+//       template <class T>
+//       __device__ T residual(const T (&x)[N], int64_t pid, int r,
+//                             const blsq_model_ctx& c) const;
+//
+// written with the operations and functions blsq_dual.cuh lists.  Without a
+// jacobian_row, the analytic kinds then derive the Jacobian row from it by
+// forward-mode dual numbers (T = blsq_dual::Dual<N>); with T = double it is
+// the residual.  An explicit jacobian_row always wins.
+//
 // The struct is default-constructed on the device and its functions must be
 // pure: the same (x, pid, r, data) gives the same bits wherever it is
 // evaluated.  c.data[k] is the k-th data tensor of the callbacks' `args`
@@ -32,7 +43,10 @@
 // operation is contracted differently where the functions are inlined, so
 // both routes evaluate the same IEEE operations on the same inputs and the
 // records agree bit for bit.  The 2-point adapter forms each quotient as
-// MODE 1 does, div_rn(f(Xp[j]) - f, dx[j], 1.0 / dx[j]).
+// MODE 1 does, div_rn(f(Xp[j]) - f, dx[j], 1.0 / dx[j]).  A derived
+// Jacobian's dual evaluation gives f as its value channel, the bits of the
+// double residual (blsq_dual.cuh), so a TRF row takes [J | f] from one
+// evaluation.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -41,6 +55,7 @@
 #include <utility>
 
 #include "../../include/blsq.h"
+#include "blsq_dual.cuh"
 #include "blsq_lin.cuh"
 
 #define BLSQ_USER_MODEL_VERSION 1
@@ -64,10 +79,51 @@ struct has_jacobian_row<
            std::declval<const blsq_model_ctx&>(), std::declval<double (&)[M::N]>()))>>
     : std::true_type {};
 
+template <class M, class = void>
+struct has_dual_residual : std::false_type {};
+template <class M>
+struct has_dual_residual<
+    M, std::enable_if_t<std::is_same<
+           blsq_dual::Dual<M::N>,
+           decltype(std::declval<const M&>().residual(
+               std::declval<const blsq_dual::Dual<M::N> (&)[M::N]>(), int64_t(), int(),
+               std::declval<const blsq_model_ctx&>()))>::value>> : std::true_type {};
+
+// where a model's Jacobian comes from: 0 none, 1 jacobian_row, 2 derived from
+// the templated residual (blsq_um_info's out[1])
+template <class M>
+constexpr int jac_source = has_jacobian_row<M>::value ? 1 : has_dual_residual<M>::value ? 2 : 0;
+
 template <int N>
 __device__ __forceinline__ void load_x(const double* __restrict__ p, double (&x)[N]) {
 #pragma unroll
     for (int k = 0; k < N; k++) x[k] = p[k];
+}
+
+// Row r of the Jacobian at x into j, from jacobian_row or from one dual
+// evaluation of the residual with x[k].d = e_k.  Returns the residual at x:
+// the dual's value channel, or the double residual after jacobian_row (left
+// unevaluated where the caller drops it).
+template <class M>
+__device__ __forceinline__ double jac_row(const M& mdl, const double (&x)[M::N], int64_t pid,
+                                          int r, const blsq_model_ctx& c, double (&j)[M::N]) {
+    constexpr int N = M::N;
+    if constexpr (jac_source<M> == 1) {
+        mdl.jacobian_row(x, pid, r, c, j);
+        return mdl.residual(x, pid, r, c);
+    } else {
+        static_assert(jac_source<M> == 2, "the model has no Jacobian");
+        blsq_dual::Dual<N> xd[N];
+#pragma unroll
+        for (int k = 0; k < N; k++) {
+            xd[k].v = x[k];
+            xd[k].d[k] = 1.0;
+        }
+        const blsq_dual::Dual<N> f = mdl.residual(xd, pid, r, c);
+#pragma unroll
+        for (int k = 0; k < N; k++) j[k] = f.d[k];
+        return f.v;
+    }
 }
 
 // MODE 3 analytic row: J at Xj (SPLIT, dogbox's bound-snapped point) or at X
@@ -86,13 +142,13 @@ struct AnalyticRows {
         if (SPLIT) {
             double xj[N];
             load_x(Xj + slot * N, xj);
-            mdl.jacobian_row(xj, pid, r, c, j);
+            jac_row(mdl, xj, pid, r, c, j);
+            a[N] = mdl.residual(x, pid, r, c);
         } else {
-            mdl.jacobian_row(x, pid, r, c, j);
+            a[N] = jac_row(mdl, x, pid, r, c, j);
         }
 #pragma unroll
         for (int k = 0; k < N; k++) a[k] = j[k];
-        a[N] = mdl.residual(x, pid, r, c);
     }
 };
 
@@ -150,7 +206,7 @@ jac_kernel(int64_t A, const int64_t* __restrict__ idx, int m, const double* __re
     const int64_t pid = idx ? idx[s] : s;
     double x[N], j[N];
     load_x(X + s * N, x);
-    M{}.jacobian_row(x, pid, r, c, j);
+    jac_row(M{}, x, pid, r, c, j);
 #pragma unroll
     for (int k = 0; k < N; k++) J[t * N + k] = j[k];
 }
@@ -187,7 +243,7 @@ int launch_lin(int64_t A, const int32_t* idx, int m, const Rows& rows, const int
 template <class M>
 int info(int* out) {
     out[0] = M::N;
-    out[1] = has_jacobian_row<M>::value ? 1 : 0;
+    out[1] = jac_source<M>;
     out[2] = BLSQ_USER_MODEL_VERSION;
     return 0;
 }
@@ -196,7 +252,7 @@ template <class M>
 int linearise(int64_t A, const int32_t* idx, int m, const double* X, const double* Xj,
               const double* const* data, int ndata, const int32_t* istate, double* lin,
               void* stream) {
-    if constexpr (!has_jacobian_row<M>::value) {
+    if constexpr (jac_source<M> == 0) {
         return BLSQ_E_UNSUPPORTED;
     } else {
         blsq_model_ctx c;
@@ -237,7 +293,7 @@ int fun(int64_t A, const int64_t* idx, int m, const double* X, const double* con
 template <class M>
 int jac(int64_t A, const int64_t* idx, int m, const double* X, const double* const* data,
         int ndata, double* J, void* stream) {
-    if constexpr (!has_jacobian_row<M>::value) {
+    if constexpr (jac_source<M> == 0) {
         return BLSQ_E_UNSUPPORTED;
     } else {
         blsq_model_ctx c;

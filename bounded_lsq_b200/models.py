@@ -165,11 +165,12 @@ def tall_callbacks(wl, lib=None):
 _PKG = os.path.dirname(os.path.abspath(__file__))
 _CSRC = os.path.join(_PKG, "csrc")
 # what a compiled model is built from besides its source: part of the cache key
-_HEADERS = [os.path.join(_CSRC, f) for f in ("blsq_user_model.cuh", "blsq_lin.cuh",
-                                             "blsq_core.cuh", "Makefile")] + \
+_HEADERS = [os.path.join(_CSRC, f) for f in ("blsq_user_model.cuh", "blsq_dual.cuh",
+                                             "blsq_lin.cuh", "blsq_core.cuh", "Makefile")] + \
            [os.path.join(_PKG, "..", "include", "blsq.h")]
 MAX_DATA = 8                              # BLSQ_MODEL_MAX_DATA
 KINDS = ("exact", "2-point", "3-point", "inlined", "inlined-2-point")
+_JACOBIAN = {0: None, 1: "analytic", 2: "autodiff"}     # blsq_um_info out[1]
 _NVCC_VERSION = {}
 _LOADED = {}
 
@@ -257,9 +258,12 @@ _UM_SIGNATURES = {
 class CompiledModel:
     """A residual model compiled by :func:`compile_model`.
 
-    ``n``: its number of parameters; ``has_jacobian``: whether it defines
-    ``jacobian_row``; ``path``: the shared object; ``built``: whether this
-    call ran nvcc (False: loaded from the cache)."""
+    ``n``: its number of parameters; ``jacobian``: where its Jacobian rows
+    come from, ``'analytic'`` (its ``jacobian_row``), ``'autodiff'`` (derived
+    from a residual templated on the scalar type by forward-mode dual
+    numbers) or None; ``has_jacobian``: ``jacobian is not None``; ``path``:
+    the shared object; ``built``: whether this call ran nvcc (False: loaded
+    from the cache)."""
 
     def __init__(self, dll, path, name, built):
         self._dll, self.path, self.name, self.built = dll, path, name, built
@@ -270,7 +274,8 @@ class CompiledModel:
         dll.blsq_um_error_string.restype = C.c_char_p
         info = (C.c_int * 3)()
         dll.blsq_um_info(info)
-        self.n, self.has_jacobian, self.version = info[0], bool(info[1]), info[2]
+        self.n, self.jacobian, self.version = info[0], _JACOBIAN[info[1]], info[2]
+        self.has_jacobian = self.jacobian is not None
 
     def _call(self, fn, *args):
         rc = getattr(self._dll, fn)(*args)
@@ -297,11 +302,12 @@ class CompiledModel:
         """(fun, jac) for ``least_squares_batched(fun, x0, jac=jac, args=data)``
         with m residuals per problem, as ``models.callbacks`` returns them:
 
-        * ``'exact'``: materialised F and J kernels (needs ``jacobian_row``);
+        * ``'exact'``: materialised F and J kernels (needs a Jacobian:
+          ``jacobian_row`` or a templated residual);
         * ``'2-point'``, ``'3-point'``: the materialised F kernel and the
           scheme's name; the solver forms the differences;
         * ``'inlined'``: the model compiled into the linearisation kernel,
-          J and f never reach HBM (needs ``jacobian_row``);
+          J and f never reach HBM (needs a Jacobian, as ``'exact'``);
         * ``'inlined-2-point'``: 2-point differences formed in registers in
           the linearisation kernel, f and the perturbed batches never reach HBM.
 
@@ -309,12 +315,18 @@ class CompiledModel:
         on the solve's device, ``PerProblem`` or shared) reach the model as
         ``blsq_model_ctx::data`` in order.  The inlined kinds serve every
         round of a dense TRF or dogbox solve; they do not take ``rows`` or
-        ``cols``."""
+        ``cols``.
+
+        A derived Jacobian (``jacobian == 'autodiff'``) is exact up to
+        rounding; TRF rows take J and f from one dual evaluation, dogbox rows
+        J from the dual at the Jacobian point and f from the double residual.
+        Both routes give the same bits, as they do with ``jacobian_row``."""
         if jac_kind not in KINDS:
             raise ValueError(f"jac_kind must be one of {KINDS}, got {jac_kind!r}")
         if jac_kind in ("exact", "inlined") and not self.has_jacobian:
-            raise ValueError(f"{self.name} defines no jacobian_row: jac_kind "
-                             f"{jac_kind!r} needs one (use '2-point' or 'inlined-2-point')")
+            raise ValueError(f"{self.name} defines no jacobian_row and its residual is not a "
+                             f"template on the scalar type: jac_kind {jac_kind!r} needs one "
+                             "of them (or use '2-point' or 'inlined-2-point')")
         m = int(m)
         if m < 1:
             raise ValueError("m must be >= 1")
